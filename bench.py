@@ -22,6 +22,8 @@ Beside the headline the line carries
 `--impl reference` times the reference's CPU path (scipy nnls per instance + the torch epilogue,
 restated in oracle/cave_oracle.py; the Python reference itself cannot travel to the GPU box) on
 all host cores on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step returned (rank 0's `loss`, `loss_i`, `grad`) as
+DIR/<name>.npy, so that two builds can be compared output for output on the same seeded inputs.
 """
 from __future__ import annotations
 
@@ -65,7 +67,36 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the `workloads` and `strong` keys")
     ap.add_argument("--cpu-sample", type=int, default=0, help="instances in the CPU baseline sample (0 = 2 x cores)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, at most 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "sweep"):
+        ap.error("--dump-outputs applies to --impl ours on a structured workload")
+    return args
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(arrays, dirname, limit=DUMP_BYTES):
+    """Write arrays as dirname/<name>.npy in float32 or float64 (other dtypes as float64).  If they exceed `limit` bytes in all,
+    the per-instance arrays (leading dimension = the batch of `grad`) keep a fixed, seeded sample of instances, whose indices
+    go to instance_index.npy."""
+    arrays = {k: a if a.dtype in (np.float32, np.float64) else a.astype(np.float64) for k, a in arrays.items()}
+    B = arrays["grad"].shape[0]
+    per_inst = [k for k, a in arrays.items() if a.ndim and a.shape[0] == B]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > limit - 4096:                  # 4 KB for the .npy headers
+        row = sum(arrays[k].nbytes // B for k in per_inst) + 8
+        keep = max(1, (limit - 4096 - (total - sum(arrays[k].nbytes for k in per_inst))) // row)
+        idx = np.sort(np.random.default_rng(0).choice(B, size=keep, replace=False))
+        arrays = {k: a[idx] if k in per_inst else a for k, a in arrays.items()}
+        arrays["instance_index"] = idx.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------- CPU reference arm
@@ -334,10 +365,10 @@ def run_ours(args):
         return info
 
     if args.workload == "sweep":
-        pts = [sweep_point(d, m, args.batch or b, max(3, args.steps // 2), rank == 0 and world == 1 and not args.no_cpu_baseline)
+        pts = [sweep_point(d, m, args.batch or b, args.steps, rank == 0 and world == 1 and not args.no_cpu_baseline)
                for d, m, b in SWEEP_FULL]
         head = next(p for p in pts if (p["d"], p["m"]) == (1225, 1024))
-        line = {"metric": METRIC, "value": head["inst_per_s"], "unit": UNIT, "n_gpus": world, "steps": max(3, args.steps // 2),
+        line = {"metric": METRIC, "value": head["inst_per_s"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
                 "warmup": 3, "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
                 "dtype": "tf32x3 Gram + f32 factor + f64 iterates", "data": "synthetic",
                 "config": {"workload": "dense projection sweep (BASELINE.json configs[4]): A ~ N(0,1)^{m x d}, exact projection, cold pack; "
@@ -357,11 +388,13 @@ def run_ours(args):
     head, A, pred, alg_bytes, gen_rows = structured(kind, batch, mode, ratio, 1, seed, want_sparse=not args.no_e2e)
     B, m_max, d = A.shape
 
+    last = {}
+
     def step():
-        return cave_forward_backward(pred, A, -1.0, mode, ratio, "mean", precision=args.precision)
+        last["out"] = cave_forward_backward(pred, A, -1.0, mode, ratio, "mean", precision=args.precision)
 
     for _ in range(max(args.warmup, 3)):
-        out = step()
+        step()
     sampler = ClockSampler(local)
     sampler.start()
     n0 = lib.cave_launch_count()
@@ -369,6 +402,8 @@ def run_ours(args):
     launches = int(lib.cave_launch_count() - n0)
     clocks = sampler.stop()
     value = B * world / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs({k: v.cpu().numpy() for k, v in last["out"].items() if not k.startswith("_")}, args.dump_outputs)
 
     # ---- per-kernel timings for the roofline (same stream, CUDA events, same inputs)
     pack = pack_constraints(A)
