@@ -276,11 +276,19 @@ int cave_pack_sparse(const int64_t* inst_off, const int64_t* row_ptr, const int3
     return pack_impl(nullptr, nullptr, B, m_max, d, pack, pack_bytes, stream, (flags & 1) != 0, &in);
 }
 
-int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
-                          double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
-                          const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
-                          int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
-                          size_t scratch_bytes, void* stream) {
+int cave_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out) {
+    if (!out) return fail(CAVE_EINVAL, "out is null");
+    if (int e = check_shape(n_instances, m_max, d)) return e;
+    *out = (size_t)n_instances * cave::warm_slot_bytes(m_max);
+    return CAVE_OK;
+}
+
+// cave_forward_backward and cave_forward_backward_warm: warm is null for the former, a checked buffer for the latter
+static int forward_backward_impl(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                                 double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                                 const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                 int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                                 size_t scratch_bytes, void* warm, size_t warm_bytes, void* stream) {
     const bool indexed = opts && opts->inst_index;
     if ((!A && !indexed) || !pred || !loss_i || !grad || !pack || !scratch) return fail(CAVE_EINVAL, "A, pred, loss_i, grad, pack, scratch must not be null");
     if (indexed && !opts->warm_pack) return fail(CAVE_EINVAL, "inst_index needs warm_pack (a pack built over the whole dataset)");
@@ -309,6 +317,12 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
     if (dense) DL = cave::make_dense_layout(B, m_max, d, dense_slots(opts, B, m_max, d), SL.total);
     const size_t need = dense ? DL.total : SL.total;
     if (scratch_bytes < need) return fail(CAVE_ENOSPC, "scratch buffer has %zu bytes, %zu needed", scratch_bytes, need);
+    if (warm) {
+        const size_t wneed = (size_t)Bpack * cave::warm_slot_bytes(m_max);
+        if (warm_bytes < wneed) return fail(CAVE_ENOSPC, "warm-start buffer has %zu bytes, %zu needed (cave_warm_bytes of %lld instances)",
+                                            warm_bytes, wneed, (long long)Bpack);
+        if (((uintptr_t)warm & 15) != 0) return fail(CAVE_EINVAL, "warm-start buffer must be 16-byte aligned");
+    }
 
     cudaStream_t st = (cudaStream_t)stream;
     if (!(opts && opts->warm_pack)) {
@@ -344,6 +358,7 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
     sp.n_packed = Bpack;
     sp.setup = (((opts && opts->warm_pack) || env_int("CAVE_COLD_SETUP", 0)) && env_int("CAVE_SETUP_CACHE", 1)) ? pb + PL.setup : nullptr;
     sp.setup_stride = PL.setup_stride;
+    sp.warm = (char*)warm; sp.warm_stride = (long long)cave::warm_slot_bytes(m_max); sp.warm_cap = (int)cave::warm_cap_v(m_max);
     sp.dense_flag = nullptr;
     if (dense) {
         // Dense regime first: instance list, then per round of n_slots instances the TF32 split, the tensor-core Gram and
@@ -408,6 +423,29 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
     g_launches += 1;
     if (ce != cudaSuccess) return fail(CAVE_ECUDA, "finalize kernel launch failed: %s", cudaGetErrorString(ce));
     return CAVE_OK;
+}
+
+int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                          double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                          const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                          int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                          size_t scratch_bytes, void* stream) {
+    return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
+                                 loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
+                                 nullptr, 0, stream);
+}
+
+int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                               double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                               const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                               int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                               size_t scratch_bytes, void* warm, size_t warm_bytes, void* stream) {
+    if (!warm) return fail(CAVE_EINVAL, "warm must not be null (use cave_forward_backward for a call without warm-start state)");
+    if (!(opts && opts->warm_pack))
+        return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
+    return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
+                                 loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
+                                 warm, warm_bytes, stream);
 }
 
 int cave_tsp_scratch_bytes(int64_t N, int32_t n_nodes, size_t* out) {

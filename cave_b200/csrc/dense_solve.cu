@@ -1042,6 +1042,7 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
             in.A = Ainst; in.gen = (const gen_t*)gen; in.ctype = p.ctype + q * p.dpad; in.avg = p.avg + q * p.dpad;
             in.d = d; in.ngen = m; in.gen_nnz = 0; in.nvalid = m; in.nsingc = 0; in.csr_ok = 0;
             in.ghash = nullptr; in.pcol = nullptr; in.pval = nullptr; in.maxl1 = 0.f; in.maxl2 = 0.f; in.setup = nullptr;
+            in.warm = nullptr; in.warm_cap = 0;
             epilogue<double, TIO, const TIO*>(cx, in, ep, c, r, p.mode != MODE_HEURISTIC, false, grad_all + (size_t)b * d,
                                               proj_all ? proj_all + (size_t)b * d : nullptr, p.loss64 + b, p.rnorm64 + b);
             if (tid == 0) { p.status[b] = status | ST_PATH_GRAM; p.iters[b] = iters; }

@@ -63,6 +63,14 @@ CAVE_HD SetupBlock make_setup_block(int64_t cap_v, int64_t cap_z, int64_t d) {
     return S;
 }
 
+// Warm-start state of a resident pack (cave_forward_backward_warm): one slot per pack instance, in a caller-owned buffer.
+//   [0]  int32 header: valid (1), nv (variables after the +- merge), tag (hash of the variable -> row map and of the
+//        sign-free flags, solver_core.cuh warm_tag), 0
+//   [16] float64 nu[cap_v]: the multipliers of the last converged Newton solve, in the solver's variable order
+// An all-zero buffer is a buffer of empty slots.  Instances with more variables than cap_v are never stored.
+CAVE_HD int64_t warm_cap_v(int64_t m_max) { return m_max < 256 ? m_max : 256; }
+CAVE_HD size_t warm_slot_bytes(int64_t m_max) { return align_up(16 + (size_t)warm_cap_v(m_max) * 8, 16); }
+
 // per-instance capacity of the packed CSR: every shipped model (TSP/VRP/SP) fits; instances that do
 // not (dense general rows) are flagged and the solver reads their rows from A instead
 CAVE_HD int64_t pack_cap_nnz(int64_t m_max, int64_t d) {

@@ -45,6 +45,9 @@ struct SolveParams {
     long long n_packed;    // instances in the pack (inst_index values must be below it)
     const char* setup;     // nullable: cached per-instance setup blocks of the pack (layout.cuh SetupBlock)
     long long setup_stride;
+    char* warm;            // nullable: warm-start slots, one per pack instance (layout.cuh warm_slot_bytes)
+    long long warm_stride;
+    int warm_cap;          // most variables a slot holds
 };
 
 struct FinalizeParams {

@@ -58,7 +58,8 @@ static __device__ __noinline__ void copy_granules(G16* dst, const G16* src, int 
 }
 #endif
 
-enum { ST_CONVERGED = 0, ST_ITER_CAP = 1, ST_STALLED = 2, ST_NOSPACE = 3, ST_SKIPPED = 4, ST_BADINPUT = 5, ST_PATH_LH = 0x100, ST_PATH_GRAM = 0x200 };
+enum { ST_CONVERGED = 0, ST_ITER_CAP = 1, ST_STALLED = 2, ST_NOSPACE = 3, ST_SKIPPED = 4, ST_BADINPUT = 5, ST_PATH_LH = 0x100, ST_PATH_GRAM = 0x200,
+       ST_WARM = 0x400 };
 enum { MODE_EXACT = 0, MODE_INNER = 1, MODE_HEURISTIC = 2 };
 
 struct SolveOpts {
@@ -347,6 +348,11 @@ struct Instance {
     float maxl1, maxl2;     // max ||a_i||_1, max ||a_i||_2^2 over the general rows
     // cached setup block of the pack (layout.cuh SetupBlock) or nullptr; its header holds the byte offsets of its arrays
     const char* setup;
+    // this instance's warm-start slot (layout.cuh warm_slot_bytes) or nullptr; it holds at most warm_cap variables.
+    // warm_from_slot = false: start from zero all the same (the cold re-solve after a failed warm start) but store the result.
+    char* warm;
+    int warm_cap;
+    bool warm_from_slot;
 };
 
 template <class T>
@@ -860,7 +866,83 @@ CAVE_DEV bool nw_setup(Ctx& cx, const Instance& in, Arena& ar, NewtonWork<T, TH,
     return true;
 }
 
-template <class T, class TH, class TC, bool HOT>
+// ------------------------------------------------------------------ warm start (layout.cuh warm_slot_bytes)
+// A slot is only ever a starting guess: another CTA of the same launch may write it while it is read (an index may hold an
+// instance twice), so nothing read from it is trusted beyond what the Newton iteration itself checks.  The helpers run
+// once per instance and are not inlined, like copy_granules, so they add nothing to the registers of the iteration.
+#ifdef CAVE_HOST_SIM
+#define CAVE_NOINLINE inline
+#else
+#define CAVE_NOINLINE static __device__ __noinline__
+#endif
+struct alignas(16) WarmHeader { int32_t valid, nv; uint32_t tag, pad; };
+
+// Hash of the variable -> row map (length and first column of every variable's row) and of the sign-free flags, computed
+// by every warp on its own (at most a few hundred variables): the same value on every thread without a barrier.
+CAVE_DEV uint32_t warm_tag(Ctx& cx, int nv, const uint8_t* vfree, const int* rptr, const int* vrow, const uint16_t* rcol) {
+    uint64_t h = 0;
+    for (int v = cx.lane; v < nv; v += Ctx::WS) {
+        const int row = vrow[v], s = rptr[row], n = rptr[row + 1] - s;
+        h += mix64(((uint64_t)v << 40) ^ ((uint64_t)vfree[v] << 36) ^ ((uint64_t)(uint32_t)n << 16) ^ (uint64_t)(n > 0 ? rcol[s] : 0));
+    }
+    h = cx.warp_sum_u64(h);
+    return (uint32_t)(h ^ (h >> 32)) ^ (uint32_t)nv;
+}
+
+// nu <- the slot's multipliers if the slot is valid for this instance (same nv and tag), with non-finite entries replaced by
+// zero and bounded variables clamped to >= 0; nu <- 0 otherwise.  Returns 1 if the slot was used (the same on every
+// thread: decided by thread 0 and broadcast through *flag, a word of shared memory, which is left at 1 or 0 accordingly).
+// Ends with a barrier.
+CAVE_NOINLINE int warm_read(Ctx cx, const char* slot, int nv, const uint8_t* vfree, const int* rptr, const int* vrow,
+                            const uint16_t* rcol, double* nu, int* flag) {
+    const uint32_t tag = warm_tag(cx, nv, vfree, rptr, vrow, rcol);
+    if (cx.tid == 0) {
+#ifdef CAVE_HOST_SIM
+        const WarmHeader h = *(const WarmHeader*)slot;
+#else
+        const int4 hv = __ldcg((const int4*)slot);
+        WarmHeader h; h.valid = hv.x; h.nv = hv.y; h.tag = (uint32_t)hv.z;
+#endif
+        *flag = (h.valid == 1 && h.nv == nv && h.tag == tag) ? 1 : 0;
+    }
+    cx.sync();
+    const int use = *flag;
+    const double* val = (const double*)(slot + sizeof(WarmHeader));
+    for (int v = cx.tid; v < nv; v += cx.nthr) {
+        double x = 0.0;
+        if (use) {
+#ifdef CAVE_HOST_SIM
+            x = val[v];
+#else
+            x = __ldcg(val + v);
+#endif
+            if (!(x - x == 0.0)) x = 0.0;                  // NaN / Inf
+            if (!vfree[v] && x < 0.0) x = 0.0;
+        }
+        nu[v] = x;
+    }
+    cx.sync();
+    return use;
+}
+
+// Stores nu as the slot's multipliers: the values first, the header after a barrier (a reader that sees the header of this
+// write and older values still only gets a starting guess).
+CAVE_NOINLINE void warm_write(Ctx cx, char* slot, int nv, const uint8_t* vfree, const int* rptr, const int* vrow,
+                              const uint16_t* rcol, const double* nu) {
+    const uint32_t tag = warm_tag(cx, nv, vfree, rptr, vrow, rcol);
+    double* val = (double*)(slot + sizeof(WarmHeader));
+    for (int v = cx.tid; v < nv; v += cx.nthr) val[v] = nu[v];
+#ifndef CAVE_HOST_SIM
+    __threadfence();
+#endif
+    cx.sync();
+    if (cx.tid == 0) {
+        WarmHeader h; h.valid = 1; h.nv = nv; h.tag = tag; h.pad = 0;
+        *(WarmHeader*)slot = h;
+    }
+}
+
+template <class T, class TH, class TC, bool HOT, bool WARM>
 CAVE_DEV void newton_solve(Ctx& cx, const Instance& in, Arena& ar, HPtr<TC, HOT> c, HPtr<T, HOT> r, T cnorm,
                            const SolveOpts& opt, Result<T>& out) {
     NewtonWork<T, TH, TC, HOT> W;
@@ -876,8 +958,15 @@ CAVE_DEV void newton_solve(Ctx& cx, const Instance& in, Arena& ar, HPtr<TC, HOT>
     const TH reg = (sizeof(TH) == 8 ? (TH)1e-11 : (TH)2e-6) * (TH)(l2max > (T)0 ? l2max : (T)1);
     const TH piv_floor = eps_mach<TH>() * (TH)(l2max > (T)0 ? l2max : (T)1);
 
-    for (int v = cx.tid; v < nv; v += cx.nthr) W.nu[v] = (T)0;
-    cx.sync();
+    // Warm start (WARM: the kernel variant launched with a warm-start buffer; without one, none of this is compiled in):
+    // nu from the instance's slot if it holds a solution of this instance.  Whether it did stays in fcnt[1] (a word of
+    // shared memory) rather than in a register live through the iteration.
+    if (WARM && in.warm && in.warm_from_slot && nv <= in.warm_cap) warm_read(cx, in.warm, nv, W.vfree.raw(), W.rptr, W.vrow, W.rcol, W.nu.raw(), W.fcnt.raw() + 1);
+    else {
+        if (WARM && in.warm && cx.tid == 0) W.fcnt[1] = 0;
+        for (int v = cx.tid; v < nv; v += cx.nthr) W.nu[v] = (T)0;
+        cx.sync();
+    }
     HPtr<T, HOT> nu = W.nu, nut = W.nut;
     const HPtr<T, HOT> rc = W.r;       // r is updated in place by every trial evaluation
     T f, dummy = (T)0;
@@ -1063,6 +1152,8 @@ CAVE_DEV void newton_solve(Ctx& cx, const Instance& in, Arena& ar, HPtr<TC, HOT>
         }
     }
     out.r = rc.raw(); out.iters = it; out.status = status;
+    if (WARM && in.warm && (int)W.fcnt[1] == 1) out.status |= ST_WARM;
+    if (WARM && in.warm && nv <= in.warm_cap && status == ST_CONVERGED) warm_write(cx, in.warm, nv, W.vfree.raw(), W.rptr, W.vrow, W.rcol, nu.raw());
 }
 
 // ------------------------------------------------------------------ Lawson-Hanson path (dense rows)
@@ -1345,7 +1436,7 @@ CAVE_DEV void epilogue(Ctx& cx, const Instance& in, const EpiParams& ep, PC c, c
 }
 
 // ------------------------------------------------------------------ one instance, start to finish
-template <class TH, class TIO, bool HOT>
+template <class TH, class TIO, bool HOT, bool WARM>
 CAVE_DEV bool solve_instance_t(Ctx& cx, const Instance& in, Arena& ar, const TIO* pred, const EpiParams& ep,
                                const SolveOpts& opt, TIO* grad_out, TIO* proj_out,
                                double* loss_out, double* rnorm_out, int* status_out, int* iters_out) {
@@ -1383,7 +1474,7 @@ CAVE_DEV bool solve_instance_t(Ctx& cx, const Instance& in, Arena& ar, const TIO
                 }
                 lh_solve<T, T>(cx, in, ar, cd, r.raw(), cnorm, opt, res);    // dense path: float64 factor in both modes
             } else {
-                newton_solve<T, TH, TIO, HOT>(cx, in, ar, c, r, cnorm, opt, res);
+                newton_solve<T, TH, TIO, HOT, WARM>(cx, in, ar, c, r, cnorm, opt, res);
             }
         } else if (solve) {
             res.status = ST_CONVERGED;      // only singleton rows: closed form, r = c
@@ -1406,18 +1497,19 @@ CAVE_DEV bool solve_instance_t(Ctx& cx, const Instance& in, Arena& ar, const TIO
 
 // One instance, start to finish.  First with the iteration's arrays pinned to shared memory (the
 // fast layout); if they do not fit (very large d or very many general rows) once more with generic
-// placement, where everything may spill to the CTA's global scratch slot.
-template <class TH, class TIO>
+// placement, where everything may spill to the CTA's global scratch slot.  WARM = false compiles none of the warm-start
+// code (Instance::warm and the fields after it are then never read).
+template <class TH, class TIO, bool WARM = false>
 CAVE_DEV void solve_instance(Ctx& cx, const Instance& in, char* smem, size_t smem_bytes, char* slot, size_t slot_bytes,
                              const TIO* pred, const EpiParams& ep, const SolveOpts& opt, TIO* grad_out, TIO* proj_out,
                              double* loss_out, double* rnorm_out, int* status_out, int* iters_out) {
     Arena ar;
     ar.init(smem, smem_bytes, slot, slot_bytes);
-    if (solve_instance_t<TH, TIO, true>(cx, in, ar, pred, ep, opt, grad_out, proj_out, loss_out, rnorm_out, status_out, iters_out))
+    if (solve_instance_t<TH, TIO, true, WARM>(cx, in, ar, pred, ep, opt, grad_out, proj_out, loss_out, rnorm_out, status_out, iters_out))
         return;
     cx.sync();
     ar.init(smem, smem_bytes, slot, slot_bytes);
-    solve_instance_t<TH, TIO, false>(cx, in, ar, pred, ep, opt, grad_out, proj_out, loss_out, rnorm_out, status_out, iters_out);
+    solve_instance_t<TH, TIO, false, WARM>(cx, in, ar, pred, ep, opt, grad_out, proj_out, loss_out, rnorm_out, status_out, iters_out);
 }
 
 }  // namespace cave

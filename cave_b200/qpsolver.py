@@ -70,12 +70,23 @@ class CavePack:
     * per dataset: pack ALL instances once (``pack_constraints(all_ctrs)``) and pass ``pack=..., index=idx``
       with ``idx[b]`` = dataset instance of batch row ``b`` — the device-resident replacement of
       DataLoader + ``collate_fn`` (src/dataset.py:133-144).  ``ctrs`` keeps the dense dataset tensor
-      resident for instances whose general rows did not fit the packed CSR (``keep_dense=False`` drops it)."""
+      resident for instances whose general rows did not fit the packed CSR (``keep_dense=False`` drops it).
+
+    ``warm`` (``warm_start=True`` at packing) is the solver state kept across calls: the multipliers of every instance's last
+    converged structured solve, from which the next call on that instance starts (``cave_forward_backward_warm`` in
+    include/cave_b200.h).  It changes where the Newton iteration starts, never what it converges to.  Calls that use one
+    pack must run on one stream, in the order they are made; ``reset_warm_start()`` empties the state."""
     buf: torch.Tensor
     shape: tuple
     data_ptr: int
     ctrs: torch.Tensor | None = None
     version: int = 0            # tensor._version of tight_ctrs when it was packed (in-place edits invalidate the pack)
+    warm: torch.Tensor | None = None    # uint8 warm-start slots, one per packed instance (None: every solve starts from zero)
+
+    def reset_warm_start(self) -> None:
+        """Forget the stored solutions (e.g. after re-initialising the predictor): the next calls start from zero."""
+        if self.warm is not None:
+            self.warm.zero_()
 
     def launch_plan(self, precision: str = "fp64", io_dtype: torch.dtype = torch.float32) -> dict:
         """Diagnostics (synchronises): the solve-kernel configuration the pack's statistics select on the device."""
@@ -94,8 +105,16 @@ class CavePack:
                 "max_hot_bytes_f64": words[3], "max_hot_bytes_f32": words[4]}
 
 
+def _warm_buffer(lib, B: int, m: int, d: int, device) -> torch.Tensor:
+    nbytes = ctypes.c_size_t()
+    _lib.check(lib.cave_warm_bytes(B, m, d, ctypes.byref(nbytes)))
+    return torch.zeros(nbytes.value, dtype=torch.uint8, device=device)
+
+
 def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = None, keep_dense: bool = True,
-                     cache_setup: bool = True) -> CavePack:
+                     cache_setup: bool = True, warm_start: bool = False) -> CavePack:
+    """``warm_start=True``: also keep the solver state across calls (``CavePack.warm``): every structured solve of an
+    instance starts from that instance's last converged solution."""
     lib = _lib.load()
     if not tight_ctrs.is_cuda:
         raise ValueError("pack_constraints expects a CUDA tensor")
@@ -110,7 +129,8 @@ def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = Non
         stream = torch.cuda.current_stream(A.device).cuda_stream
         _lib.check(lib.cave_pack_ex(_ptr(A), _ptr(m_rows), B, m, d, 1 if cache_setup else 0, _ptr(buf), nbytes.value,
                                     ctypes.c_void_p(stream)))
-    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version))
+    warm = _warm_buffer(lib, B, m, d, A.device) if warm_start else None
+    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version), warm)
 
 
 @dataclass
@@ -175,10 +195,12 @@ class SparseConstraints:
                                  self.m_max, self.d)
 
 
-def pack_constraints_sparse(sc: SparseConstraints, device=None, cache_setup: bool = True) -> CavePack:
+def pack_constraints_sparse(sc: SparseConstraints, device=None, cache_setup: bool = True,
+                            warm_start: bool = False) -> CavePack:
     """Builds the device-resident pack straight from per-instance CSR (``cave_pack_sparse``): no dense tensor exists on
     the device, so instances that would need it (no singleton row at all, or general rows beyond the packed-CSR
-    capacity) report ``CAVE_ST_NOSPACE``.  Host tensors are uploaded on the current stream (pinned -> asynchronous)."""
+    capacity) report ``CAVE_ST_NOSPACE``.  Host tensors are uploaded on the current stream (pinned -> asynchronous).
+    ``warm_start``: as for ``pack_constraints``."""
     lib = _lib.load()
     dev = _device_of(sc.val, device)
     B, m, d = sc.batch, int(sc.m_max), int(sc.d)
@@ -193,7 +215,17 @@ def pack_constraints_sparse(sc: SparseConstraints, device=None, cache_setup: boo
         stream = torch.cuda.current_stream(dev).cuda_stream
         _lib.check(lib.cave_pack_sparse(_ptr(io), _ptr(rp), _ptr(col), _ptr(val), B, m, d, 1 if cache_setup else 0,
                                         _ptr(buf), nbytes.value, ctypes.c_void_p(stream)))
-    return CavePack(buf, (B, m, d), 0, None, 0)
+    warm = _warm_buffer(lib, B, m, d, dev) if warm_start else None
+    return CavePack(buf, (B, m, d), 0, None, 0, warm)
+
+
+def _call_forward_backward(lib, pack: CavePack | None, *args) -> None:
+    """cave_forward_backward, or cave_forward_backward_warm with the pack's warm-start state when it has one."""
+    if pack is not None and pack.warm is not None:
+        *head, stream = args
+        _lib.check(lib.cave_forward_backward_warm(*head, _ptr(pack.warm), pack.warm.numel(), stream))
+    else:
+        _lib.check(lib.cave_forward_backward(*args))
 
 
 def cave_forward_backward(pred_cost: torch.Tensor, tight_ctrs: torch.Tensor, sign: float, mode: int,
@@ -263,11 +295,11 @@ def cave_forward_backward(pred_cost: torch.Tensor, tight_ctrs: torch.Tensor, sig
         m_rows = _to_device(m_rows, dev, torch.int32)
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(lib.cave_forward_backward(
-            _ptr(A), _ptr(m_rows), _ptr(pred), B, m, d, float(sign), int(mode), float(inner_ratio),
+        _call_forward_backward(
+            lib, pack, _ptr(A), _ptr(m_rows), _ptr(pred), B, m, d, float(sign), int(mode), float(inner_ratio),
             _lib.REDUCE[reduction], _lib.F64 if io_dtype == torch.float64 else _lib.F32, compute,
             ctypes.byref(opts), _ptr(loss), _ptr(loss_i), _ptr(grad), _ptr(proj), _ptr(rnorm), _ptr(status),
-            _ptr(iters), _ptr(pack_buf), pack_buf.numel(), _ptr(scratch), scratch.numel(), ctypes.c_void_p(stream)))
+            _ptr(iters), _ptr(pack_buf), pack_buf.numel(), _ptr(scratch), scratch.numel(), ctypes.c_void_p(stream))
     out = dict(loss=loss_i if reduction == "none" else loss, loss_i=loss_i, grad=grad)
     if want_proj:
         out["proj"], out["rnorm"] = proj, rnorm
@@ -314,11 +346,11 @@ def _forward_backward_indexed(lib, pred_cost, ctrs, sign, mode, inner_ratio, red
     iters = torch.empty(B, dtype=torch.int32, device=dev) if want_status else None
     with torch.cuda.device(dev):
         stream = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(lib.cave_forward_backward(
-            _ptr(A), None, _ptr(pred), B, m, d, float(sign), int(mode), float(inner_ratio),
+        _call_forward_backward(
+            lib, pack, _ptr(A), None, _ptr(pred), B, m, d, float(sign), int(mode), float(inner_ratio),
             _lib.REDUCE[reduction], _lib.F64 if io_dtype == torch.float64 else _lib.F32, compute,
             ctypes.byref(opts), _ptr(loss), _ptr(loss_i), _ptr(grad), _ptr(proj), _ptr(rnorm), _ptr(status),
-            _ptr(iters), _ptr(pack.buf), pack.buf.numel(), _ptr(scratch), scratch.numel(), ctypes.c_void_p(stream)))
+            _ptr(iters), _ptr(pack.buf), pack.buf.numel(), _ptr(scratch), scratch.numel(), ctypes.c_void_p(stream))
     out = dict(loss=loss_i if reduction == "none" else loss, loss_i=loss_i, grad=grad)
     if want_proj:
         out["proj"], out["rnorm"] = proj, rnorm

@@ -65,6 +65,8 @@ extern "C" {
 #define CAVE_ST_BADINPUT 5      /* NaN / Inf in the prediction: no solve, outputs are NaN  */
 #define CAVE_ST_PATH_LH 0x100   /* flag: solved by the Lawson-Hanson path (else Newton)    */
 #define CAVE_ST_PATH_GRAM 0x200 /* flag: solved by the dense path (tensor-core Gram + Gram-space Newton) */
+#define CAVE_ST_WARM 0x400      /* flag: the Newton solve started from the instance's warm-start slot
+                                   (cave_forward_backward_warm; never set without one)              */
 
 typedef struct cave_solver_opts {
     int32_t max_iter;        /* Newton iterations / LH pivots cap; <= 0 -> default (200 / 3*m) */
@@ -171,6 +173,33 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
                           int32_t* status, int32_t* iters,
                           void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
                           void* stream);
+
+/* Warm start of a resident pack.  The structured Newton solve of pack instance q normally starts from nu = 0; with a
+ * warm-start buffer it starts from the multipliers of q's last converged solve, which the call stores back.  The buffer
+ * holds one fixed-size slot per pack instance (a header and at most min(m_max, 256) float64 multipliers); an all-zero
+ * buffer is a buffer of empty slots, so a reset is a memset.  cave_warm_bytes(): bytes for n_instances (the n_packed of
+ * an indexed call, B otherwise).
+ * cave_forward_backward_warm(): cave_forward_backward plus the buffer (device pointer, 16-byte aligned).  It needs
+ * opts->warm_pack = 1 (CAVE_EINVAL otherwise) and warm_bytes >= cave_warm_bytes() (CAVE_ENOSPC otherwise).  The slot of
+ * batch row b is inst_index[b], or b without an index.
+ *  - A slot is used only if it holds a solution for the same variables (count and a hash of the structure); its values
+ *    are a starting guess (non-finite entries become 0, bounded ones are clamped to >= 0).  Such instances report
+ *    CAVE_ST_WARM.  If a warm start ends CAVE_ST_ITER_CAP or CAVE_ST_STALLED, the instance is solved once more from zero
+ *    in the same call (iters is the sum; CAVE_ST_WARM is then clear): a warm start never ends worse than a cold one.
+ *  - A slot is written only by a structured (Newton) instance that ends CAVE_ST_CONVERGED.  Lawson-Hanson and dense-path
+ *    instances, heuristic mode, empty cones, NaN / Inf predictions and instances with more variables than a slot holds
+ *    leave it untouched.
+ *  - Calls that share one buffer must be ordered (one stream), as calls that share a pack or scratch are.  An index may
+ *    hold an instance twice: the slot is then read and written concurrently, which can only change the starting guess. */
+int cave_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out);
+int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred,
+                               int64_t B, int64_t m_max, int64_t d,
+                               double sign, int mode, double inner_ratio, int reduction,
+                               int io_dtype, int compute_dtype, const cave_solver_opts* opts,
+                               void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                               int32_t* status, int32_t* iters,
+                               void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
+                               void* warm, size_t warm_bytes, void* stream);
 
 /* Diagnostic for the dense regime (north_star item 1): runs cave_pack() on A and then only the TF32 split and the
  * tensor-core Gram kernel (TMA tiles -> tcgen05.mma, 3xTF32, float32 accumulation in TMEM) for the first
