@@ -14,12 +14,13 @@ MODE_EXACT, MODE_INNER, MODE_HEURISTIC = 0, 1, 2
 REDUCE = {"mean": 0, "sum": 1, "none": 2}
 F32, F64 = 0, 1
 ST_CONVERGED, ST_ITER_CAP, ST_STALLED, ST_NOSPACE, ST_SKIPPED, ST_BADINPUT, ST_PATH_LH, ST_PATH_GRAM = 0, 1, 2, 3, 4, 5, 0x100, 0x200
-ST_WARM = 0x400     # flag: the Newton solve started from the pack's warm-start state
+ST_WARM = 0x400     # flag: the (structured or dense) Newton solve started from the pack's warm-start state
 
 EXPORTS = ("cave_abi_version", "cave_last_error", "cave_get_limits", "cave_pack_bytes",
            "cave_scratch_bytes", "cave_pack", "cave_forward_backward", "cave_plan_offset", "cave_plan_choice",
            "cave_dense_gram", "cave_launch_count", "cave_dense_ctrl_offset", "cave_pack_sparse",
-           "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm")
+           "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm",
+           "cave_dense_warm_bytes", "cave_forward_backward_warm_ex")
 
 
 class SolverOpts(ctypes.Structure):
@@ -66,7 +67,12 @@ def load() -> ctypes.CDLL:
     lib.cave_forward_backward_warm.argtypes = [P, P, P, I64, I64, I64, F, I32, F, I32, I32, I32,
                                                ctypes.POINTER(SolverOpts), P, P, P, P, P, P, P,
                                                P, ctypes.c_size_t, P, ctypes.c_size_t, P, ctypes.c_size_t, P]
+    lib.cave_forward_backward_warm_ex.argtypes = [P, P, P, I64, I64, I64, F, I32, F, I32, I32, I32,
+                                                  ctypes.POINTER(SolverOpts), P, P, P, P, P, P, P,
+                                                  P, ctypes.c_size_t, P, ctypes.c_size_t, P, ctypes.c_size_t,
+                                                  P, ctypes.c_size_t, P]
     lib.cave_warm_bytes.argtypes = [I64, I64, I64, SZP]
+    lib.cave_dense_warm_bytes.argtypes = [I64, I64, I64, SZP]
     lib.cave_dense_gram.argtypes = [P, I64, I64, I64, ctypes.POINTER(SolverOpts), P, P, P, ctypes.c_size_t, P, ctypes.c_size_t, P]
     lib.cave_tsp_scratch_bytes.argtypes = [I64, I32, SZP]
     lib.cave_tsp_solve.argtypes = [P, I64, I32, P, P, P, ctypes.c_size_t, P]
@@ -77,7 +83,8 @@ def load() -> ctypes.CDLL:
     lib.cave_plan_choice.argtypes = [ctypes.POINTER(ctypes.c_uint64), I64, I32, I32, IP, IP, IP]
     for name in ("cave_get_limits", "cave_pack_bytes", "cave_scratch_bytes", "cave_pack", "cave_forward_backward",
                  "cave_plan_offset", "cave_plan_choice", "cave_dense_gram", "cave_dense_ctrl_offset", "cave_pack_sparse",
-                 "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm"):
+                 "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm",
+                 "cave_dense_warm_bytes", "cave_forward_backward_warm_ex"):
         getattr(lib, name).restype = I32
     _lib = lib
     return lib

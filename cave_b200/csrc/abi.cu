@@ -283,12 +283,21 @@ int cave_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out) 
     return CAVE_OK;
 }
 
-// cave_forward_backward and cave_forward_backward_warm: warm is null for the former, a checked buffer for the latter
+int cave_dense_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out) {
+    if (!out) return fail(CAVE_EINVAL, "out is null");
+    if (int e = check_shape(n_instances, m_max, d)) return e;
+    *out = (size_t)n_instances * cave::dense_warm_slot_bytes(m_max);
+    return CAVE_OK;
+}
+
+// cave_forward_backward and its warm-start variants: warm / warm_dense are null for the former, checked buffers (either
+// may be null) for the latter
 static int forward_backward_impl(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
                                  double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
                                  const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
                                  int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
-                                 size_t scratch_bytes, void* warm, size_t warm_bytes, void* stream) {
+                                 size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense,
+                                 size_t warm_dense_bytes, void* stream) {
     const bool indexed = opts && opts->inst_index;
     if ((!A && !indexed) || !pred || !loss_i || !grad || !pack || !scratch) return fail(CAVE_EINVAL, "A, pred, loss_i, grad, pack, scratch must not be null");
     if (indexed && !opts->warm_pack) return fail(CAVE_EINVAL, "inst_index needs warm_pack (a pack built over the whole dataset)");
@@ -322,6 +331,13 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         if (warm_bytes < wneed) return fail(CAVE_ENOSPC, "warm-start buffer has %zu bytes, %zu needed (cave_warm_bytes of %lld instances)",
                                             warm_bytes, wneed, (long long)Bpack);
         if (((uintptr_t)warm & 15) != 0) return fail(CAVE_EINVAL, "warm-start buffer must be 16-byte aligned");
+    }
+    if (warm_dense) {
+        const size_t wneed = (size_t)Bpack * cave::dense_warm_slot_bytes(m_max);
+        if (warm_dense_bytes < wneed)
+            return fail(CAVE_ENOSPC, "dense warm-start buffer has %zu bytes, %zu needed (cave_dense_warm_bytes of %lld instances)",
+                        warm_dense_bytes, wneed, (long long)Bpack);
+        if (((uintptr_t)warm_dense & 15) != 0) return fail(CAVE_EINVAL, "dense warm-start buffer must be 16-byte aligned");
     }
 
     cudaStream_t st = (cudaStream_t)stream;
@@ -374,6 +390,7 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         dp.grad = grad; dp.proj = proj; dp.loss64 = sp.loss64; dp.rnorm64 = sp.rnorm64; dp.status = sp.status; dp.iters = sp.iters;
         dp.mode = mode; dp.inner_ratio = inner_ratio; dp.sign = sign; dp.gscale = sp.gscale;
         dp.max_iter = 0; dp.max_ls = sp.max_ls; dp.tol = sp.tol; dp.io_f32 = io_dtype == CAVE_F32; dp.nk = (int)(DL.d_pad / 32);
+        dp.warm = (char*)warm_dense; dp.warm_stride = (long long)cave::dense_warm_slot_bytes(m_max); dp.warm_cap = (int)cave::dense_warm_cap(m_max);
         ce = cave::launch_dense_list(dp, st);
         g_launches += 1;
         if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense list kernel launch failed: %s", cudaGetErrorString(ce));
@@ -432,7 +449,7 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
                           size_t scratch_bytes, void* stream) {
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 nullptr, 0, stream);
+                                 nullptr, 0, nullptr, 0, stream);
 }
 
 int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -445,7 +462,22 @@ int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void
         return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, stream);
+                                 warm, warm_bytes, nullptr, 0, stream);
+}
+
+int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                                  double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                                  const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                  int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                                  size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                  void* stream) {
+    if (!warm && !warm_dense)
+        return fail(CAVE_EINVAL, "warm and warm_dense must not both be null (use cave_forward_backward for a call without warm-start state)");
+    if (!(opts && opts->warm_pack))
+        return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
+    return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
+                                 loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, stream);
 }
 
 int cave_tsp_scratch_bytes(int64_t N, int32_t n_nodes, size_t* out) {

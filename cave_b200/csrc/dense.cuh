@@ -100,6 +100,9 @@ struct DenseParams {
     int io_f32;
     int nk;                     // d_pad / 32
     int tc_update;              // set by launch_dense_solve: the Cholesky block-column update runs on the tensor cores (shared memory permitting)
+    char* warm;                 // nullable: warm-start slots, one per pack instance (layout.cuh dense_warm_slot_bytes)
+    long long warm_stride;
+    int warm_cap;               // most rows a slot holds
 };
 
 cudaError_t launch_dense_list(const DenseParams& p, cudaStream_t stream);

@@ -748,6 +748,59 @@ __device__ __noinline__ void chol_blocked_o(float* W, int ldw, int nf, float flo
     chol_blocked<TC>(W, ldw, nf, floor_, S, tid);
 }
 
+// ---- Warm start (layout.cuh dense_warm_slot_bytes).  As for the structured solve (solver_core.cuh warm_read), a slot is
+// only ever a starting guess: an index may hold an instance twice, so another CTA may write a slot while it is read.  The
+// helpers run once per instance, outside the iteration, and are outlined with by-value arguments like the phases above.
+// Hash of m and of every general row's index and length, by one warp (every lane gets the value).
+__device__ uint32_t dense_warm_tag(const int4* gen, int m, int lane) {
+    uint64_t h = 0;
+    for (int v = lane; v < m; v += 32) {
+        const int4 gv = gen[v];
+        h += mix64(((uint64_t)v << 40) ^ ((uint64_t)(uint32_t)gv.y << 20) ^ (uint64_t)(uint32_t)gv.x);
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) h += __shfl_xor_sync(0xffffffffu, h, o);
+    return (uint32_t)(h ^ (h >> 32)) ^ (uint32_t)m;
+}
+// lam[0, m) <- the slot's multipliers if the slot holds a solution of this instance (same m and tag), with non-finite values
+// replaced by 0 and negative ones clamped to 0; lam is left as it is otherwise.  Returns the slot's flags, or -1 if it was
+// not used: the same on every thread (decided by thread 0, broadcast through *word, a word of shared memory).  All threads
+// call; ends with a barrier.
+__device__ __noinline__ int dense_warm_read(const char* slot, const int4* gen, int m, double* lam, int* word) {
+    const int tid = threadIdx.x;
+    if (tid < 32) {
+        const uint32_t tag = dense_warm_tag(gen, m, tid);
+        if (tid == 0) {
+            const int4 h = __ldcg((const int4*)slot);
+            *word = (h.x == 1 && h.y == m && (uint32_t)h.z == tag) ? (h.w & 1) : -1;
+        }
+    }
+    __syncthreads();
+    const int flags = *word;
+    if (flags >= 0) {
+        const double* val = (const double*)(slot + 16);
+        for (int v = tid; v < m; v += kDT) {
+            double x = __ldcg(val + v);
+            if (!(x - x == 0.0) || x < 0.0) x = 0.0;        // NaN / Inf, negative
+            lam[v] = x;
+        }
+    }
+    __syncthreads();
+    return flags;
+}
+// Stores lam[0, m) and flags as the slot's solution: the values first, the header after a fence and a barrier (a reader that
+// sees the new header with older values still only gets a starting guess).  All threads call.
+__device__ __noinline__ void dense_warm_write(char* slot, const int4* gen, int m, const double* lam, int flags) {
+    const int tid = threadIdx.x;
+    double* val = (double*)(slot + 16);
+    for (int v = tid; v < m; v += kDT) val[v] = lam[v];
+    uint32_t tag = 0;
+    if (tid < 32) tag = dense_warm_tag(gen, m, tid);
+    __threadfence();
+    __syncthreads();
+    if (tid == 0) *(int4*)slot = make_int4(1, m, (int)tag, flags);
+}
+
 // Coarse phase clocks (thread 0, clock64 deltas summed over instances): only in -DCAVE_DENSE_PROFILE builds.
 #ifdef CAVE_DENSE_PROFILE
 #define DPROF_BEGIN() long long dprof_t = clock64()
@@ -760,8 +813,9 @@ enum { DP_SETUP = 0, DP_KKT = 1, DP_FREESET = 2, DP_GATHER = 3, DP_CHOL = 4, DP_
        DP_TRUEGRAD = 8, DP_EPILOGUE = 9, DP_SWITCH = 10, DP_NFACT = 11, DP_NITER = 12 };
 
 // TC: the Cholesky block-column update runs on the tensor cores (a separate instantiation, so that the register allocation of
-// each variant only sees the update it uses).
-template <class TIO, bool TC>
+// each variant only sees the update it uses).  WARM: the variant for calls with a warm-start buffer (p.warm); the other one
+// compiles none of the warm-start code.
+template <class TIO, bool TC, bool WARM>
 __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
     extern __shared__ __align__(16) char dsm[];
     __shared__ double red[64];
@@ -882,22 +936,36 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
             // Tikhonov term above the accuracy of G~ (3xTF32 operands, truncating float32 accumulation: ~1.5e-5 relative on the
             // diagonal at d = 1225), so that the factored matrix is positive definite even where G_FF is singular (|F| > d)
             const float regf = (float)(4e-5 * dmax), floorf_ = (float)(1e-6 * dmax);
-            int nf_fact = -1;                           // size of the free set the factor in W belongs to (-1: none)
-            double f = 0.0;                             // phase 1: q(lam);  phase 2: 1/2 ||r||^2
-            int phase = 1, since_best = 0, it1 = 0, it2 = 0;
-            double res_best = 1e300;
+            // Warm start: lam from the instance's slot if it holds a solution of this instance.  Such a start skips the
+            // Gram-space phase (it would pull lam towards the float32-accurate optimum of G~, while the stored lam is anchored
+            // to A) and resumes with the metric the stored solve ended with.
+            char* wslot = (WARM && p.warm && m <= p.warm_cap) ? p.warm + q * (size_t)p.warm_stride : nullptr;
+            bool warm_try = false;
+            const bool scaled0 = scaled;
+            if (WARM && wslot) {
+                const int wf = dense_warm_read(wslot, gen, m, S.lam, &s_nf);
+                warm_try = wf >= 0;
+                if (warm_try) scaled = (wf & 1) != 0;
+            }
             double* lam = S.lam; double* lamt = S.lamt; double* g = S.g; double* gt = S.gt;
             double* rc = r; double* rtr = rt;
+            for (;;) {      // (WARM: a failed warm start is solved once more from zero; otherwise one pass)
+            int nf_fact = -1;                           // size of the free set the factor in W belongs to (-1: none)
+            double f = 0.0;                             // phase 1: q(lam);  phase 2: 1/2 ||r||^2
+            int phase = 1, since_best = 0, it1 = (WARM && warm_try) ? max_it1 : 0, it2 = 0;     // (a warm start switches at once)
+            double res_best = 1e300;
             status = ST_ITER_CAP;
             for (;;) {
                 double res = kkt_residual(lam, g, m, cx);
                 DPROF(DP_KKT);
                 if (phase == 1 && (res <= tolG || it1 >= max_it1)) {
-                    if (res > 1e-4 * scale) { handed_back = true; why = 1; why_phase = 1; break; }       // the Gram-space iteration did not settle
+                    if (res > 1e-4 * scale && !(WARM && warm_try)) { handed_back = true; why = 1; why_phase = 1; break; }       // the Gram-space iteration did not settle
                     // ---- switch to the true problem: r = c - A^T lam, g = -A r
                     phase = 2; since_best = 0; res_best = 1e300;
                     f = 0.5 * (OUT_RES ? true_residual_o<TIO>(Ainst, d, m, lam, c, rc, S.sup, S.arow, red, &s_cnt)
                                                   : true_residual<TIO>(Ainst, d, m, lam, c, rc, S, cx, &s_cnt));
+                    // a warm point that fits worse than lam = 0 (or overflows) is not worth starting from
+                    if (WARM && warm_try && !(f <= 0.5 * cc)) { status = ST_STALLED; break; }
                     if (OUT_GRAD) true_gradient_o(Ainst, d, m, rc, g, S.arow, red); else true_gradient(Ainst, d, m, rc, g, S, cx);
                     res = kkt_residual(lam, g, m, cx);
                     DPROF(DP_SWITCH);
@@ -1026,10 +1094,23 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
                 __syncthreads();
             }
             __syncthreads();
+            if (!(WARM && warm_try && (handed_back || status == ST_ITER_CAP || status == ST_STALLED))) break;
+            // ---- the warm start failed: back to the state the setup above left (iterations add up; only this cold
+            // solve may hand the instance back to Lawson-Hanson)
+            warm_try = false; handed_back = false; why = 0; why_phase = 0; scaled = scaled0;
+            lam = S.lam; lamt = S.lamt; g = S.g; gt = S.gt; rc = r; rtr = rt;
+            for (int k = tid; k < d; k += kDT) r[k] = (double)c[k];
+            for (int v = tid; v < mp; v += kDT) {
+                S.lam[v] = 0.0; S.lamt[v] = 0.0; S.g[v] = v < m ? -bsrc[v] : 0.0; S.gt[v] = 0.0; S.dir[v] = 0.0;
+            }
+            __syncthreads();
+            }
             if (!handed_back && rc != r) {          // the epilogue reads r
                 for (int k = tid; k < d; k += kDT) r[k] = rc[k];
             }
             __syncthreads();
+            if (WARM && wslot && !handed_back && status == ST_CONVERGED) dense_warm_write(wslot, gen, m, lam, scaled ? 1 : 0);
+            if (WARM && warm_try) status |= ST_WARM;
         }
         if (handed_back && p.no_handback) { handed_back = false; status |= (why << 16) | (why_phase << 12); }
         if (handed_back) {
@@ -1076,8 +1157,11 @@ cudaError_t launch_dense_solve(const DenseParams& p_in, cudaStream_t stream) {
         const size_t want = smem + (size_t)atoi(e_pad);
         smem = want < budget ? want : budget;
     }
-    void (*kern)(DenseParams) = p.tc_update ? (p.io_f32 ? dense_solve_kernel<float, true> : dense_solve_kernel<double, true>)
-                                            : (p.io_f32 ? dense_solve_kernel<float, false> : dense_solve_kernel<double, false>);
+    void (*kern)(DenseParams) =
+        p.warm ? (p.tc_update ? (p.io_f32 ? dense_solve_kernel<float, true, true> : dense_solve_kernel<double, true, true>)
+                              : (p.io_f32 ? dense_solve_kernel<float, false, true> : dense_solve_kernel<double, false, true>))
+               : (p.tc_update ? (p.io_f32 ? dense_solve_kernel<float, true, false> : dense_solve_kernel<double, true, false>)
+                              : (p.io_f32 ? dense_solve_kernel<float, false, false> : dense_solve_kernel<double, false, false>));
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int dev = 0, sms = 148;

@@ -70,6 +70,14 @@ CAVE_HD SetupBlock make_setup_block(int64_t cap_v, int64_t cap_z, int64_t d) {
 // An all-zero buffer is a buffer of empty slots.  Instances with more variables than cap_v are never stored.
 CAVE_HD int64_t warm_cap_v(int64_t m_max) { return m_max < 256 ? m_max : 256; }
 CAVE_HD size_t warm_slot_bytes(int64_t m_max) { return align_up(16 + (size_t)warm_cap_v(m_max) * 8, 16); }
+// Warm-start state of the dense Gram-space Newton solve (cave_forward_backward_warm_ex), a second caller-owned buffer with
+// one slot per pack instance:
+//   [0]  int32 header: valid (1), m (general rows), tag (hash of m and of every row's index and length, dense_solve.cu
+//        dense_warm_tag), flags (bit 0: the solve ended with the diagonal metric)
+//   [16] float64 lam[cap]: the multipliers of the last converged dense solve, in the instance's general-row order
+// An all-zero buffer is a buffer of empty slots.  The dense path takes at most 2048 rows, so every dense instance fits.
+CAVE_HD int64_t dense_warm_cap(int64_t m_max) { return m_max < 2048 ? m_max : 2048; }
+CAVE_HD size_t dense_warm_slot_bytes(int64_t m_max) { return align_up(16 + (size_t)dense_warm_cap(m_max) * 8, 16); }
 
 // per-instance capacity of the packed CSR: every shipped model (TSP/VRP/SP) fits; instances that do
 // not (dense general rows) are flagged and the solver reads their rows from A instead

@@ -75,18 +75,23 @@ class CavePack:
     ``warm`` (``warm_start=True`` at packing) is the solver state kept across calls: the multipliers of every instance's last
     converged structured solve, from which the next call on that instance starts (``cave_forward_backward_warm`` in
     include/cave_b200.h).  It changes where the Newton iteration starts, never what it converges to.  Calls that use one
-    pack must run on one stream, in the order they are made; ``reset_warm_start()`` empties the state."""
+    pack must run on one stream, in the order they are made; ``reset_warm_start()`` empties the state.
+
+    ``warm_dense`` (``warm_dense=True`` as well) does the same for instances solved by the dense Gram-space Newton path
+    (``cave_forward_backward_warm_ex``): 8 bytes per general row and instance, which a structured dataset never uses."""
     buf: torch.Tensor
     shape: tuple
     data_ptr: int
     ctrs: torch.Tensor | None = None
     version: int = 0            # tensor._version of tight_ctrs when it was packed (in-place edits invalidate the pack)
     warm: torch.Tensor | None = None    # uint8 warm-start slots, one per packed instance (None: every solve starts from zero)
+    warm_dense: torch.Tensor | None = None  # uint8 slots of the dense path (None: dense-path solves start from zero)
 
     def reset_warm_start(self) -> None:
         """Forget the stored solutions (e.g. after re-initialising the predictor): the next calls start from zero."""
-        if self.warm is not None:
-            self.warm.zero_()
+        for buf in (self.warm, self.warm_dense):
+            if buf is not None:
+                buf.zero_()
 
     def launch_plan(self, precision: str = "fp64", io_dtype: torch.dtype = torch.float32) -> dict:
         """Diagnostics (synchronises): the solve-kernel configuration the pack's statistics select on the device."""
@@ -105,16 +110,19 @@ class CavePack:
                 "max_hot_bytes_f64": words[3], "max_hot_bytes_f32": words[4]}
 
 
-def _warm_buffer(lib, B: int, m: int, d: int, device) -> torch.Tensor:
+def _warm_buffer(sizer, B: int, m: int, d: int, device) -> torch.Tensor:
     nbytes = ctypes.c_size_t()
-    _lib.check(lib.cave_warm_bytes(B, m, d, ctypes.byref(nbytes)))
+    _lib.check(sizer(B, m, d, ctypes.byref(nbytes)))
     return torch.zeros(nbytes.value, dtype=torch.uint8, device=device)
 
 
 def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = None, keep_dense: bool = True,
-                     cache_setup: bool = True, warm_start: bool = False) -> CavePack:
+                     cache_setup: bool = True, warm_start: bool = False, warm_dense: bool = False) -> CavePack:
     """``warm_start=True``: also keep the solver state across calls (``CavePack.warm``): every structured solve of an
-    instance starts from that instance's last converged solution."""
+    instance starts from that instance's last converged solution.  ``warm_dense=True`` (with ``warm_start=True``): the
+    same for the dense Gram-space path (``CavePack.warm_dense``)."""
+    if warm_dense and not warm_start:
+        raise ValueError("warm_dense=True needs warm_start=True")
     lib = _lib.load()
     if not tight_ctrs.is_cuda:
         raise ValueError("pack_constraints expects a CUDA tensor")
@@ -129,8 +137,9 @@ def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = Non
         stream = torch.cuda.current_stream(A.device).cuda_stream
         _lib.check(lib.cave_pack_ex(_ptr(A), _ptr(m_rows), B, m, d, 1 if cache_setup else 0, _ptr(buf), nbytes.value,
                                     ctypes.c_void_p(stream)))
-    warm = _warm_buffer(lib, B, m, d, A.device) if warm_start else None
-    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version), warm)
+    warm = _warm_buffer(lib.cave_warm_bytes, B, m, d, A.device) if warm_start else None
+    wdense = _warm_buffer(lib.cave_dense_warm_bytes, B, m, d, A.device) if warm_dense else None
+    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version), warm, wdense)
 
 
 @dataclass
@@ -215,13 +224,18 @@ def pack_constraints_sparse(sc: SparseConstraints, device=None, cache_setup: boo
         stream = torch.cuda.current_stream(dev).cuda_stream
         _lib.check(lib.cave_pack_sparse(_ptr(io), _ptr(rp), _ptr(col), _ptr(val), B, m, d, 1 if cache_setup else 0,
                                         _ptr(buf), nbytes.value, ctypes.c_void_p(stream)))
-    warm = _warm_buffer(lib, B, m, d, dev) if warm_start else None
+    warm = _warm_buffer(lib.cave_warm_bytes, B, m, d, dev) if warm_start else None
     return CavePack(buf, (B, m, d), 0, None, 0, warm)
 
 
 def _call_forward_backward(lib, pack: CavePack | None, *args) -> None:
-    """cave_forward_backward, or cave_forward_backward_warm with the pack's warm-start state when it has one."""
-    if pack is not None and pack.warm is not None:
+    """cave_forward_backward, or cave_forward_backward_warm(_ex) with the pack's warm-start state when it has one."""
+    if pack is not None and pack.warm_dense is not None:
+        *head, stream = args
+        nwarm = pack.warm.numel() if pack.warm is not None else 0
+        _lib.check(lib.cave_forward_backward_warm_ex(*head, _ptr(pack.warm), nwarm, _ptr(pack.warm_dense),
+                                                     pack.warm_dense.numel(), stream))
+    elif pack is not None and pack.warm is not None:
         *head, stream = args
         _lib.check(lib.cave_forward_backward_warm(*head, _ptr(pack.warm), pack.warm.numel(), stream))
     else:

@@ -65,8 +65,9 @@ extern "C" {
 #define CAVE_ST_BADINPUT 5      /* NaN / Inf in the prediction: no solve, outputs are NaN  */
 #define CAVE_ST_PATH_LH 0x100   /* flag: solved by the Lawson-Hanson path (else Newton)    */
 #define CAVE_ST_PATH_GRAM 0x200 /* flag: solved by the dense path (tensor-core Gram + Gram-space Newton) */
-#define CAVE_ST_WARM 0x400      /* flag: the Newton solve started from the instance's warm-start slot
-                                   (cave_forward_backward_warm; never set without one)              */
+#define CAVE_ST_WARM 0x400      /* flag: the Newton solve (structured, or dense with CAVE_ST_PATH_GRAM) started from the
+                                   instance's warm-start slot (cave_forward_backward_warm / _warm_ex;
+                                   never set without one)                                           */
 
 typedef struct cave_solver_opts {
     int32_t max_iter;        /* Newton iterations / LH pivots cap; <= 0 -> default (200 / 3*m) */
@@ -200,6 +201,32 @@ int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void
                                int32_t* status, int32_t* iters,
                                void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
                                void* warm, size_t warm_bytes, void* stream);
+
+/* Warm start of the dense Gram-space Newton solve (CAVE_ST_PATH_GRAM), with a second buffer of the same kind: one slot per
+ * pack instance, a 16-byte header (valid, m, a hash of the rows' indices and lengths, and whether the solve ended with the
+ * diagonal metric) and at most min(m_max, 2048) float64 multipliers lambda in the instance's general-row order; all zero =
+ * all empty.  cave_dense_warm_bytes(): bytes for n_instances, as cave_warm_bytes().
+ * cave_forward_backward_warm_ex(): cave_forward_backward_warm plus warm_dense.  Either buffer may be null, not both
+ * (CAVE_EINVAL); it needs opts->warm_pack = 1 (CAVE_EINVAL); each buffer must be 16-byte aligned (CAVE_EINVAL) and hold
+ * the pack's instances (CAVE_ENOSPC).  The structured solve uses warm as above; a null warm_dense keeps the dense path cold.
+ *  - A dense instance whose slot holds a solution for the same rows starts from it (non-finite and negative values become
+ *    0), skips the Gram-space phase and iterates on the true problem at once; it reports CAVE_ST_WARM.  If that ends
+ *    CAVE_ST_ITER_CAP or CAVE_ST_STALLED, would hand the instance back to Lawson-Hanson, or starts from a point that fits
+ *    worse than lambda = 0, the instance is solved once more from zero in the same call (iters is the sum; CAVE_ST_WARM is
+ *    then clear).  Only that cold solve may hand the instance back.
+ *  - A slot is written only by a dense instance that ends CAVE_ST_CONVERGED on the dense path.  Instances handed back,
+ *    Lawson-Hanson and structured instances, heuristic mode (no dense path) and NaN / Inf predictions leave it untouched.
+ *  - Ordering and duplicate indices: as for warm. */
+int cave_dense_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out);
+int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const void* pred,
+                                  int64_t B, int64_t m_max, int64_t d,
+                                  double sign, int mode, double inner_ratio, int reduction,
+                                  int io_dtype, int compute_dtype, const cave_solver_opts* opts,
+                                  void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                  int32_t* status, int32_t* iters,
+                                  void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
+                                  void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                  void* stream);
 
 /* Diagnostic for the dense regime (north_star item 1): runs cave_pack() on A and then only the TF32 split and the
  * tensor-core Gram kernel (TMA tiles -> tcgen05.mma, 3xTF32, float32 accumulation in TMEM) for the first
