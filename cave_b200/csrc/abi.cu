@@ -297,7 +297,7 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
                                  const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
                                  int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
                                  size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense,
-                                 size_t warm_dense_bytes, void* stream) {
+                                 size_t warm_dense_bytes, const void* gram, size_t gram_bytes, void* stream) {
     const bool indexed = opts && opts->inst_index;
     if ((!A && !indexed) || !pred || !loss_i || !grad || !pack || !scratch) return fail(CAVE_EINVAL, "A, pred, loss_i, grad, pack, scratch must not be null");
     if (indexed && !opts->warm_pack) return fail(CAVE_EINVAL, "inst_index needs warm_pack (a pack built over the whole dataset)");
@@ -338,6 +338,14 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
             return fail(CAVE_ENOSPC, "dense warm-start buffer has %zu bytes, %zu needed (cave_dense_warm_bytes of %lld instances)",
                         warm_dense_bytes, wneed, (long long)Bpack);
         if (((uintptr_t)warm_dense & 15) != 0) return fail(CAVE_EINVAL, "dense warm-start buffer must be 16-byte aligned");
+    }
+    if (gram) {
+        if (!A) return fail(CAVE_EINVAL, "a Gram cache needs A (the dense path reads the rows of A)");
+        if (((uintptr_t)gram & 15) != 0) return fail(CAVE_EINVAL, "Gram cache must be 16-byte aligned");
+        const size_t gneed = cave::gram_cache_bytes(Bpack, 0, m_max);
+        if (gram_bytes < gneed)
+            return fail(CAVE_ENOSPC, "Gram cache has %zu bytes, at least %zu needed (cave_gram_cache_bytes of %lld instances)",
+                        gram_bytes, gneed, (long long)Bpack);
     }
 
     cudaStream_t st = (cudaStream_t)stream;
@@ -391,6 +399,8 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         dp.mode = mode; dp.inner_ratio = inner_ratio; dp.sign = sign; dp.gscale = sp.gscale;
         dp.max_iter = 0; dp.max_ls = sp.max_ls; dp.tol = sp.tol; dp.io_f32 = io_dtype == CAVE_F32; dp.nk = (int)(DL.d_pad / 32);
         dp.warm = (char*)warm_dense; dp.warm_stride = (long long)cave::dense_warm_slot_bytes(m_max); dp.warm_cap = (int)cave::dense_warm_cap(m_max);
+        // with the pack's Gram cache the prep kernel writes no TF32 planes and the Gram kernel is not launched
+        dp.gram = (const char*)gram; dp.gram_bytes = gram_bytes;
         ce = cave::launch_dense_list(dp, st);
         g_launches += 1;
         if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense list kernel launch failed: %s", cudaGetErrorString(ce));
@@ -399,10 +409,12 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
             dp.round = (int)r;
             ce = cave::launch_dense_prep(dp, st);
             if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense prep kernel launch failed: %s", cudaGetErrorString(ce));
-            ce = cave::launch_dense_gram(dp, st);
-            if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense Gram kernel launch failed: %s (%s)", cudaGetErrorString(ce), cave::dense_last_error());
+            if (!gram) {
+                ce = cave::launch_dense_gram(dp, st);
+                if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense Gram kernel launch failed: %s (%s)", cudaGetErrorString(ce), cave::dense_last_error());
+            }
             ce = cave::launch_dense_solve(dp, st);
-            g_launches += 3;
+            g_launches += gram ? 2 : 3;
             if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense solve kernel launch failed: %s", cudaGetErrorString(ce));
         }
         sp.dense_flag = (const int*)(sb + DL.flag);
@@ -449,7 +461,7 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
                           size_t scratch_bytes, void* stream) {
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 nullptr, 0, nullptr, 0, stream);
+                                 nullptr, 0, nullptr, 0, nullptr, 0, stream);
 }
 
 int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -462,7 +474,7 @@ int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void
         return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, nullptr, 0, stream);
+                                 warm, warm_bytes, nullptr, 0, nullptr, 0, stream);
 }
 
 int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -477,7 +489,113 @@ int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const v
         return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, warm_dense, warm_dense_bytes, stream);
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, nullptr, 0, stream);
+}
+
+int cave_forward_backward_resident(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                                   double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                                   const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                   int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                                   size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                   const void* gram, size_t gram_bytes, void* stream) {
+    if (!warm && !warm_dense && !gram)
+        return fail(CAVE_EINVAL, "warm, warm_dense and gram must not all be null (use cave_forward_backward for a call without them)");
+    if (!(opts && opts->warm_pack))
+        return fail(CAVE_EINVAL, "warm-start state and Gram cache need opts->warm_pack = 1: they belong to a pack built beforehand by cave_pack()");
+    return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
+                                 loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, gram, gram_bytes, stream);
+}
+
+int cave_gram_cache_bytes(int64_t N, int64_t n_cached, int64_t m_max, int64_t d, size_t* out) {
+    if (!out) return fail(CAVE_EINVAL, "out is null");
+    if (int e = check_shape(N, m_max, d)) return e;
+    if (n_cached < 0 || n_cached > N) return fail(CAVE_EINVAL, "n_cached = %lld must be in [0, N = %lld]", (long long)n_cached, (long long)N);
+    *out = cave::gram_cache_bytes(N, n_cached, m_max);
+    return CAVE_OK;
+}
+
+int cave_gram_cache_count(const void* pack, size_t pack_bytes, int64_t N, int64_t m_max, int64_t d, int32_t* n_cached_dev,
+                          void* stream) {
+    if (!pack || !n_cached_dev) return fail(CAVE_EINVAL, "pack and n_cached_dev must not be null");
+    if (int e = check_shape(N, m_max, d)) return e;
+    const cave::PackLayout PL = cave::make_pack_layout(N, m_max, d);
+    if (pack_bytes < PL.total) return fail(CAVE_ENOSPC, "pack buffer has %zu bytes, %zu needed", pack_bytes, PL.total);
+    if (((uintptr_t)pack & 255) != 0) return fail(CAVE_EINVAL, "pack must be 256-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t ce;
+    static const float kSomeA = 0.f;
+    cave_solver_opts o;
+    memset(&o, 0, sizeof(o));
+    o.dense_mode = 1;
+    if (!dense_enabled(&o, &kSomeA, m_max, d, CAVE_MODE_EXACT)) {
+        ce = cudaMemsetAsync(n_cached_dev, 0, 4, st);       // a shape the dense path never takes: nothing to cache
+    } else {
+        const char* pb = (const char*)pack;
+        ce = cave::launch_gram_cache_map((const int*)(pb + PL.nvalid), (const int*)(pb + PL.ngen), (const int*)(pb + PL.nsingc),
+                                         (int)N, (int)cave::dense_m_pad(m_max), nullptr, n_cached_dev, nullptr, st);
+        g_launches += 1;
+    }
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "Gram cache count failed: %s", cudaGetErrorString(ce));
+    return CAVE_OK;
+}
+
+int cave_gram_cache_build(const float* A, int64_t N, int64_t m_max, int64_t d, const cave_solver_opts* opts, void* cache,
+                          size_t cache_bytes, const void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
+                          void* stream) {
+    if (!A || !cache || !pack || !scratch) return fail(CAVE_EINVAL, "A, cache, pack, scratch must not be null");
+    if (int e = check_shape(N, m_max, d)) return e;
+    cave_solver_opts o;
+    memset(&o, 0, sizeof(o));
+    if (opts) o = *opts;
+    o.dense_mode = 1; o.inst_index = nullptr; o.n_packed = 0;
+    if (!dense_enabled(&o, A, m_max, d, CAVE_MODE_EXACT)) return fail(CAVE_ELIMIT, "shape outside the dense path (128 <= m_max <= 2048)");
+    if (((uintptr_t)scratch & 255) != 0 || ((uintptr_t)pack & 255) != 0) return fail(CAVE_EINVAL, "pack and scratch must be 256-byte aligned");
+    if (((uintptr_t)cache & 15) != 0) return fail(CAVE_EINVAL, "Gram cache must be 16-byte aligned");
+    const size_t cneed = cave::gram_cache_bytes(N, 0, m_max);
+    if (cache_bytes < cneed)
+        return fail(CAVE_ENOSPC, "Gram cache has %zu bytes, at least %zu needed (cave_gram_cache_bytes of %lld instances)",
+                    cache_bytes, cneed, (long long)N);
+    const cave::PackLayout PL = cave::make_pack_layout(N, m_max, d);
+    if (pack_bytes < PL.total) return fail(CAVE_ENOSPC, "pack buffer has %zu bytes, %zu needed", pack_bytes, PL.total);
+    const ScratchPlan SPn = plan_scratch(&o, N, m_max, d);
+    const cave::ScratchLayout SL = cave::make_scratch_layout(N, d, SPn.cr, SPn.cz, 8, SPn.n_slots, SPn.n_large, SPn.large_bytes, SPn.small_bytes);
+    const cave::DenseLayout DL = cave::make_dense_layout(N, m_max, d, dense_slots(&o, N, m_max, d), SL.total);
+    if (scratch_bytes < DL.total) return fail(CAVE_ENOSPC, "scratch buffer has %zu bytes, %zu needed", scratch_bytes, DL.total);
+    const char* pb = (const char*)pack;
+    char* cb = (char*)cache;
+    cudaStream_t st = (cudaStream_t)stream;
+    // slots the buffer holds: a buffer sized for fewer instances than the pack has stays invalid (header valid = 0)
+    const long long cap = (long long)((cache_bytes - cave::gram_cache_base(N)) / ((size_t)DL.m_pad * DL.m_pad * 4));
+    cave::DenseParams dp;
+    memset(&dp, 0, sizeof(dp));
+    dp.A = A; dp.B = (int)N; dp.m_max = (int)m_max; dp.d = (int)d; dp.n_packed = N;
+    dp.nvalid = (const int*)(pb + PL.nvalid); dp.ngen = (const int*)(pb + PL.ngen); dp.nsingc = (const int*)(pb + PL.nsingc);
+    dp.gen = (const int4*)(pb + PL.gen); dp.ctype = (const unsigned char*)(pb + PL.ctype); dp.avg = (const float*)(pb + PL.avg);
+    dp.dpad = PL.dpad; dp.ws = (char*)scratch; dp.L = DL; dp.force = 1; dp.trace_b = -1; dp.sign = 0.0; dp.io_f32 = 1; dp.nk = (int)(DL.d_pad / 32);
+    dp.pred = A;       // prep also forms b = A c: any finite data will do (as in cave_dense_gram)
+    cudaError_t ce = cave::launch_gram_cache_map(dp.nvalid, dp.ngen, dp.nsingc, (int)N, (int)DL.m_pad, (int*)(cb + 16), nullptr,
+                                                 (int*)cb, st);
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "Gram cache map kernel launch failed: %s", cudaGetErrorString(ce));
+    ce = cave::launch_dense_list(dp, st);
+    g_launches += 2;
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense list kernel launch failed: %s", cudaGetErrorString(ce));
+    // the same list -> prep -> Gram sequence as a call (dense_mode = 1, every pack instance), round by round
+    const int64_t rounds = (N + DL.n_slots - 1) / DL.n_slots;
+    for (int64_t r = 0; r < rounds; ++r) {
+        dp.round = (int)r;
+        ce = cave::launch_dense_prep(dp, st);
+        if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense prep kernel launch failed: %s", cudaGetErrorString(ce));
+        ce = cave::launch_dense_gram(dp, st);
+        if (ce != cudaSuccess) return fail(CAVE_ECUDA, "dense Gram kernel launch failed: %s (%s)", cudaGetErrorString(ce), cave::dense_last_error());
+        ce = cave::launch_gram_cache_copy(dp, cb, cap, st);
+        g_launches += 3;
+        if (ce != cudaSuccess) return fail(CAVE_ECUDA, "Gram cache copy kernel launch failed: %s", cudaGetErrorString(ce));
+    }
+    ce = cave::launch_gram_cache_seal(cb, cap, st);
+    g_launches += 1;
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "Gram cache seal kernel launch failed: %s", cudaGetErrorString(ce));
+    return CAVE_OK;
 }
 
 int cave_tsp_scratch_bytes(int64_t N, int32_t n_nodes, size_t* out) {

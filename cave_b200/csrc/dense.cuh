@@ -62,6 +62,28 @@ CAVE_HD DenseLayout make_dense_layout(int64_t B, int64_t m_max, int64_t d, int64
     return L;
 }
 
+// Gram cache of a resident dataset (cave_gram_cache_build), a caller-owned buffer over the N instances of a pack:
+//   [0]     int32 header: valid (1 once every slot is written), n_cached, m_pad, N
+//   [16]    int32 map[N]: cache slot of pack instance q, or -1 (instances the dense path can never take)
+//   [base]  float32 G~[n_cached][m_pad][m_pad], base = gram_cache_base(N): each slot in the layout of a DenseLayout::G slot
+//           (both triangles), zero outside the instance's leading (128-row block) square
+// Which instances get a slot is decided by dense_qualifies() with force semantics, so every instance that any call puts on the
+// dense path has one.
+CAVE_HD size_t gram_cache_base(int64_t N) { return align_up(16 + (size_t)N * 4, 1024); }
+CAVE_HD size_t gram_cache_bytes(int64_t N, int64_t n_cached, int64_t m_max) {
+    const size_t mp = (size_t)dense_m_pad(m_max);
+    return gram_cache_base(N) + (size_t)n_cached * mp * mp * 4;
+}
+
+// The dense-path criterion of one pack instance (dense_list_kernel and the Gram cache): no singleton row, every valid row a
+// general row, at least kDenseMinRows of them, and (unless forced) not far more rows than columns.  The m_pad <= 2048 bound
+// is a property of the shape and is checked on the host.
+__device__ __forceinline__ bool dense_qualifies(const int* nvalid, const int* ngen, const int* nsingc, long long q, int force,
+                                                int d) {
+    const int ng = ngen[q];
+    return nsingc[q] == 0 && ng >= kDenseMinRows && nvalid[q] == ng && (force || ng <= d + d / 2);
+}
+
 // tiles of the upper block triangle of an nI x nI block matrix (128-row blocks), 128 x (128 | 256) each
 CAVE_HD int dense_tiles(int nI) {
     int t = 0;
@@ -103,6 +125,8 @@ struct DenseParams {
     char* warm;                 // nullable: warm-start slots, one per pack instance (layout.cuh dense_warm_slot_bytes)
     long long warm_stride;
     int warm_cap;               // most rows a slot holds
+    const char* gram;           // nullable: the pack's Gram cache (gram_cache_bytes); prep then writes no planes, the Gram
+    size_t gram_bytes;          // kernel is not launched and the solve reads G~ from the instance's cache slot
 };
 
 cudaError_t launch_dense_list(const DenseParams& p, cudaStream_t stream);
@@ -110,5 +134,13 @@ cudaError_t launch_dense_prep(const DenseParams& p, cudaStream_t stream);
 cudaError_t launch_dense_gram(const DenseParams& p, cudaStream_t stream);
 cudaError_t launch_dense_solve(const DenseParams& p, cudaStream_t stream);
 const char* dense_last_error();
+// Gram cache build (gram_kernel.cu).  map: the cache slot of every pack instance that dense_qualifies() with force, or -1,
+// into map (nullable) and their number into *n_cached; header (nullable): also {0, n_cached, m_pad, N} there.
+cudaError_t launch_gram_cache_map(const int* nvalid, const int* ngen, const int* nsingc, int N, int m_pad, int* map,
+                                  int* n_cached, int* header, cudaStream_t stream);
+// copies G~ of this round's slots (p.round, inst_index null) to their cache slots; slots at or beyond cap are skipped
+cudaError_t launch_gram_cache_copy(const DenseParams& p, char* cache, long long cap, cudaStream_t stream);
+// header valid = 1 if n_cached <= cap
+cudaError_t launch_gram_cache_seal(char* cache, long long cap, cudaStream_t stream);
 
 }  // namespace cave

@@ -814,8 +814,9 @@ enum { DP_SETUP = 0, DP_KKT = 1, DP_FREESET = 2, DP_GATHER = 3, DP_CHOL = 4, DP_
 
 // TC: the Cholesky block-column update runs on the tensor cores (a separate instantiation, so that the register allocation of
 // each variant only sees the update it uses).  WARM: the variant for calls with a warm-start buffer (p.warm); the other one
-// compiles none of the warm-start code.
-template <class TIO, bool TC, bool WARM>
+// compiles none of the warm-start code.  GC: the variant for calls with a Gram cache (p.gram), which reads G~ from the
+// instance's cache slot instead of the round's DenseLayout::G slot.
+template <class TIO, bool TC, bool WARM, bool GC>
 __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
     extern __shared__ __align__(16) char dsm[];
     __shared__ double red[64];
@@ -886,6 +887,19 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
         const float* Ainst = p.A + q * (size_t)p.m_max * d;
         const int4* gen = p.gen + q * (size_t)p.m_max;
         const float* G = (const float*)(p.ws + p.L.G) + (size_t)s * mp * mp;
+        bool gram_ok = true;
+        if constexpr (GC) {
+            // The cache comes from outside the library: it must describe this pack (header valid, same m_pad and N, a slot
+            // count that fits its bytes) and hold a slot for q.  Otherwise the instance reports CAVE_ST_BADINPUT, and G keeps
+            // pointing at the (unused, in-bounds) slot of the round so that the setup below reads nothing out of bounds.
+            const int4 h = *(const int4*)p.gram;
+            const size_t base = gram_cache_base(p.n_packed), slot_bytes = (size_t)mp * mp * 4;
+            const long long ncap = (long long)((p.gram_bytes - base) / slot_bytes);
+            const int slot = ((const int*)(p.gram + 16))[q];
+            gram_ok = h.x == 1 && h.z == mp && (long long)h.w == p.n_packed && h.y >= 0 && (long long)h.y <= ncap &&
+                      slot >= 0 && slot < h.y;
+            if (gram_ok) G = (const float*)(p.gram + base + (size_t)slot * slot_bytes);
+        }
         float* W = (float*)(p.ws + p.L.W) + (size_t)s * mp * mp;
         const double* bsrc = (const double*)(p.ws + p.L.bvec) + (size_t)s * mp;
         const float* l1src = (const float*)(p.ws + p.L.l1) + (size_t)s * mp;
@@ -922,7 +936,8 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
         // when a line search has to cut the step to the order of 1 / G_vv (the signature of the identity scaling overshooting).
         bool scaled = osum * 0.25 < 0.25 * dsum;
         const double cnorm = sqrt(cc);
-        const bool finite_in = cc < 1e300 && !(p.mode != MODE_EXACT && p.plan && p.plan[PLAN_NO_AVG] != 0ull);   // (or a pack without the average in a mode that needs it)
+        const bool finite_in = cc < 1e300 && !(p.mode != MODE_EXACT && p.plan && p.plan[PLAN_NO_AVG] != 0ull)    // (or a pack without the average in a mode that needs it,
+                               && (!GC || gram_ok);                                                         //  or a Gram cache without this instance)
         DPROF(DP_SETUP);
         int status = ST_BADINPUT, iters = 0;
         bool handed_back = false;
@@ -1141,6 +1156,12 @@ __global__ void __launch_bounds__(kDT, 1) dense_solve_kernel(DenseParams p) {
     }
 }
 
+template <class TIO, bool TC>
+static void (*dense_solve_variant(const DenseParams& p))(DenseParams) {
+    return p.warm ? (p.gram ? dense_solve_kernel<TIO, TC, true, true> : dense_solve_kernel<TIO, TC, true, false>)
+                  : (p.gram ? dense_solve_kernel<TIO, TC, false, true> : dense_solve_kernel<TIO, TC, false, false>);
+}
+
 cudaError_t launch_dense_solve(const DenseParams& p_in, cudaStream_t stream) {
     DenseParams p = p_in;
     // static shared memory of the kernel (reduction scratch, counters, mbarrier): 1.6 KB
@@ -1158,10 +1179,8 @@ cudaError_t launch_dense_solve(const DenseParams& p_in, cudaStream_t stream) {
         smem = want < budget ? want : budget;
     }
     void (*kern)(DenseParams) =
-        p.warm ? (p.tc_update ? (p.io_f32 ? dense_solve_kernel<float, true, true> : dense_solve_kernel<double, true, true>)
-                              : (p.io_f32 ? dense_solve_kernel<float, false, true> : dense_solve_kernel<double, false, true>))
-               : (p.tc_update ? (p.io_f32 ? dense_solve_kernel<float, true, false> : dense_solve_kernel<double, true, false>)
-                              : (p.io_f32 ? dense_solve_kernel<float, false, false> : dense_solve_kernel<double, false, false>));
+        p.tc_update ? (p.io_f32 ? dense_solve_variant<float, true>(p) : dense_solve_variant<double, true>(p))
+                    : (p.io_f32 ? dense_solve_variant<float, false>(p) : dense_solve_variant<double, false>(p));
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return e;
     int dev = 0, sms = 148;

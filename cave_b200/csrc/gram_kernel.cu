@@ -45,8 +45,7 @@ __global__ void __launch_bounds__(1024) dense_list_kernel(DenseParams p) {
         if (b < p.B && p.mode != 2) {
             const long long q = p.inst_index ? (long long)p.inst_index[b] : (long long)b;
             if (q >= 0 && q < p.n_packed) {           // (out-of-range indices are reported by the general kernel)
-                const int ng = p.ngen[q];
-                take = p.nsingc[q] == 0 && ng >= kDenseMinRows && p.nvalid[q] == ng && (p.force || ng <= p.d + p.d / 2);
+                take = dense_qualifies(p.nvalid, p.ngen, p.nsingc, q, p.force, p.d);
             }
         }
         const unsigned m = __ballot_sync(0xffffffffu, take);
@@ -70,8 +69,9 @@ cudaError_t launch_dense_list(const DenseParams& p, cudaStream_t stream) {
 }
 
 // ------------------------------------------------------------------ prep: TF32 split, b = A c, row 1-norms
+// PLANES = false (calls with a Gram cache): the same loop without the plane stores, so b and ||a_i||_1 are bit-identical.
 
-template <class TIO>
+template <class TIO, bool PLANES>
 __global__ void __launch_bounds__(256) dense_prep_kernel(DenseParams p) {
     const int* ctrl = (const int*)(p.ws + p.L.ctrl);
     const int* list = (const int*)(p.ws + p.L.list);
@@ -107,9 +107,11 @@ __global__ void __launch_bounds__(256) dense_prep_kernel(DenseParams p) {
         for (int u = 0; u < 4; ++u) {
             const int k = k0 + u * 32 + lane;
             if (k < d_pad) {
-                const float h = tf32_rn(x[u]);
-                hi[k] = h;
-                lo[k] = tf32_rn(x[u] - h);
+                if constexpr (PLANES) {
+                    const float h = tf32_rn(x[u]);
+                    hi[k] = h;
+                    lo[k] = tf32_rn(x[u] - h);
+                }
                 dot += (double)x[u] * (double)(TIO)(p.sign * (double)c[u]);
                 l1 += fabsf(x[u]);
             }
@@ -125,8 +127,84 @@ __global__ void __launch_bounds__(256) dense_prep_kernel(DenseParams p) {
 
 cudaError_t launch_dense_prep(const DenseParams& p, cudaStream_t stream) {
     const unsigned grid = (unsigned)(p.L.n_slots * (p.L.m_pad / 8));
-    if (p.io_f32) dense_prep_kernel<float><<<grid, 256, 0, stream>>>(p);
-    else dense_prep_kernel<double><<<grid, 256, 0, stream>>>(p);
+    if (p.gram) {
+        if (p.io_f32) dense_prep_kernel<float, false><<<grid, 256, 0, stream>>>(p);
+        else dense_prep_kernel<double, false><<<grid, 256, 0, stream>>>(p);
+    } else {
+        if (p.io_f32) dense_prep_kernel<float, true><<<grid, 256, 0, stream>>>(p);
+        else dense_prep_kernel<double, true><<<grid, 256, 0, stream>>>(p);
+    }
+    return cudaGetLastError();
+}
+
+// ------------------------------------------------------------------ Gram cache of a resident dataset (dense.cuh)
+// One CTA: ordered compaction of the pack instances the dense path could take (dense_qualifies with force semantics).
+__global__ void __launch_bounds__(1024) gram_cache_map_kernel(const int* nvalid, const int* ngen, const int* nsingc, int N,
+                                                              int m_pad, int* map, int* n_cached, int* header) {
+    __shared__ int wsum[32];
+    __shared__ int base_s;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (threadIdx.x == 0) base_s = 0;
+    __syncthreads();
+    for (int q0 = 0; q0 < N; q0 += 1024) {
+        const int q = q0 + threadIdx.x;
+        const bool take = q < N && dense_qualifies(nvalid, ngen, nsingc, q, 1, 0);
+        const unsigned m = __ballot_sync(0xffffffffu, take);
+        if (lane == 0) wsum[warp] = __popc(m);
+        __syncthreads();
+        int off = base_s;
+        for (int w = 0; w < warp; ++w) off += wsum[w];
+        if (map && q < N) map[q] = take ? off + __popc(m & ((1u << lane) - 1u)) : -1;
+        __syncthreads();
+        if (threadIdx.x == 0) { int t = 0; for (int w = 0; w < 32; ++w) t += wsum[w]; base_s += t; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        if (n_cached) *n_cached = base_s;
+        if (header) { header[0] = 0; header[1] = base_s; header[2] = m_pad; header[3] = N; }
+    }
+}
+
+cudaError_t launch_gram_cache_map(const int* nvalid, const int* ngen, const int* nsingc, int N, int m_pad, int* map,
+                                  int* n_cached, int* header, cudaStream_t stream) {
+    gram_cache_map_kernel<<<1, 1024, 0, stream>>>(nvalid, ngen, nsingc, N, m_pad, map, n_cached, header);
+    return cudaGetLastError();
+}
+
+// One warp per row of a slot, grid as dense_prep_kernel: the instance's leading square of G~ is copied, the rest of the
+// cache slot is zeroed (those entries of a DenseLayout::G slot are never written).
+__global__ void __launch_bounds__(256) gram_cache_copy_kernel(DenseParams p, char* cache, long long cap) {
+    const int* ctrl = (const int*)(p.ws + p.L.ctrl);
+    const int* list = (const int*)(p.ws + p.L.list);
+    const int m_pad = (int)p.L.m_pad;
+    const int chunks = m_pad / 8;
+    const int s = blockIdx.x / chunks;
+    const int j = p.round * (int)p.L.n_slots + s;
+    if (j >= ctrl[0]) return;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int row = (blockIdx.x - s * chunks) * 8 + warp;
+    const int q = list[j];
+    const int slot = ((const int*)(cache + 16))[q];
+    if (slot < 0 || slot >= cap) return;
+    const int lim = (p.ngen[q] + 127) & ~127;
+    const float4* src = (const float4*)((const float*)(p.ws + p.L.G) + ((size_t)s * m_pad + row) * m_pad);
+    float4* dst = (float4*)((float*)(cache + gram_cache_base(p.n_packed)) + ((size_t)slot * m_pad + row) * m_pad);
+    for (int c = lane; c < m_pad / 4; c += 32)
+        dst[c] = (row < lim && 4 * c < lim) ? src[c] : make_float4(0.f, 0.f, 0.f, 0.f);
+}
+
+cudaError_t launch_gram_cache_copy(const DenseParams& p, char* cache, long long cap, cudaStream_t stream) {
+    const unsigned grid = (unsigned)(p.L.n_slots * (p.L.m_pad / 8));
+    gram_cache_copy_kernel<<<grid, 256, 0, stream>>>(p, cache, cap);
+    return cudaGetLastError();
+}
+
+__global__ void gram_cache_seal_kernel(int* header, long long cap) {
+    if (header[1] <= cap) header[0] = 1;
+}
+
+cudaError_t launch_gram_cache_seal(char* cache, long long cap, cudaStream_t stream) {
+    gram_cache_seal_kernel<<<1, 1, 0, stream>>>((int*)cache, cap);
     return cudaGetLastError();
 }
 

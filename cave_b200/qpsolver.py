@@ -78,7 +78,11 @@ class CavePack:
     pack must run on one stream, in the order they are made; ``reset_warm_start()`` empties the state.
 
     ``warm_dense`` (``warm_dense=True`` as well) does the same for instances solved by the dense Gram-space Newton path
-    (``cave_forward_backward_warm_ex``): 8 bytes per general row and instance, which a structured dataset never uses."""
+    (``cave_forward_backward_warm_ex``): 8 bytes per general row and instance, which a structured dataset never uses.
+
+    ``gram`` (``cache_gram=True`` at packing) holds G~ = A Aᵀ of every instance the dense path could take, computed once by
+    the same tensor-core kernel a call runs (``cave_gram_cache_build``); calls with the pack then skip the TF32 split and the
+    Gram kernel and give bit-identical results.  It is constant data, not solver state: ``reset_warm_start()`` keeps it."""
     buf: torch.Tensor
     shape: tuple
     data_ptr: int
@@ -86,6 +90,7 @@ class CavePack:
     version: int = 0            # tensor._version of tight_ctrs when it was packed (in-place edits invalidate the pack)
     warm: torch.Tensor | None = None    # uint8 warm-start slots, one per packed instance (None: every solve starts from zero)
     warm_dense: torch.Tensor | None = None  # uint8 slots of the dense path (None: dense-path solves start from zero)
+    gram: torch.Tensor | None = None    # uint8 Gram cache (None: every call computes G~ of its dense instances)
 
     def reset_warm_start(self) -> None:
         """Forget the stored solutions (e.g. after re-initialising the predictor): the next calls start from zero."""
@@ -117,12 +122,17 @@ def _warm_buffer(sizer, B: int, m: int, d: int, device) -> torch.Tensor:
 
 
 def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = None, keep_dense: bool = True,
-                     cache_setup: bool = True, warm_start: bool = False, warm_dense: bool = False) -> CavePack:
+                     cache_setup: bool = True, warm_start: bool = False, warm_dense: bool = False,
+                     cache_gram: bool = False) -> CavePack:
     """``warm_start=True``: also keep the solver state across calls (``CavePack.warm``): every structured solve of an
     instance starts from that instance's last converged solution.  ``warm_dense=True`` (with ``warm_start=True``): the
-    same for the dense Gram-space path (``CavePack.warm_dense``)."""
+    same for the dense Gram-space path (``CavePack.warm_dense``).  ``cache_gram=True``: compute G~ = A Aᵀ of every
+    instance the dense path could take once, here (``CavePack.gram``, m_pad² · 4 bytes per such instance, m_pad = m
+    rounded up to 128; ``None`` if there is none); later calls with the pack reuse it."""
     if warm_dense and not warm_start:
         raise ValueError("warm_dense=True needs warm_start=True")
+    if cache_gram and not keep_dense:
+        raise ValueError("cache_gram=True needs keep_dense=True: the dense path reads the rows of the dataset tensor")
     lib = _lib.load()
     if not tight_ctrs.is_cuda:
         raise ValueError("pack_constraints expects a CUDA tensor")
@@ -139,7 +149,32 @@ def pack_constraints(tight_ctrs: torch.Tensor, m_rows: torch.Tensor | None = Non
                                     ctypes.c_void_p(stream)))
     warm = _warm_buffer(lib.cave_warm_bytes, B, m, d, A.device) if warm_start else None
     wdense = _warm_buffer(lib.cave_dense_warm_bytes, B, m, d, A.device) if warm_dense else None
-    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version), warm, wdense)
+    gram = _gram_cache(lib, A, buf) if cache_gram else None
+    return CavePack(buf, (B, m, d), A.data_ptr(), A if keep_dense else None, int(tight_ctrs._version), warm, wdense, gram)
+
+
+def _gram_cache(lib, A: torch.Tensor, pack_buf: torch.Tensor) -> torch.Tensor | None:
+    """The Gram cache of a packed dataset (None if no instance can take the dense path).  Reads the number of cached
+    instances back once (a synchronisation) to size the buffer."""
+    N, m, d = A.shape
+    dev = A.device
+    with torch.cuda.device(dev):
+        stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        cnt = torch.zeros(1, dtype=torch.int32, device=dev)
+        _lib.check(lib.cave_gram_cache_count(_ptr(pack_buf), pack_buf.numel(), N, m, d, _ptr(cnt), stream))
+        n_cached = int(cnt.item())
+        if n_cached == 0:
+            return None
+        nb = ctypes.c_size_t()
+        _lib.check(lib.cave_gram_cache_bytes(N, n_cached, m, d, ctypes.byref(nb)))
+        gram = torch.zeros(nb.value, dtype=torch.uint8, device=dev)
+        # one round per SM: the Gram kernel's grid is one CTA per SM, and the scratch stays small
+        opts = _opts(dense=True, dense_slots=torch.cuda.get_device_properties(dev).multi_processor_count)
+        _lib.check(lib.cave_scratch_bytes(N, m, d, _lib.F64, ctypes.byref(opts), ctypes.byref(nb)))
+        scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)
+        _lib.check(lib.cave_gram_cache_build(_ptr(A), N, m, d, ctypes.byref(opts), _ptr(gram), gram.numel(), _ptr(pack_buf),
+                                             pack_buf.numel(), _ptr(scratch), scratch.numel(), stream))
+    return gram
 
 
 @dataclass
@@ -229,8 +264,15 @@ def pack_constraints_sparse(sc: SparseConstraints, device=None, cache_setup: boo
 
 
 def _call_forward_backward(lib, pack: CavePack | None, *args) -> None:
-    """cave_forward_backward, or cave_forward_backward_warm(_ex) with the pack's warm-start state when it has one."""
-    if pack is not None and pack.warm_dense is not None:
+    """cave_forward_backward, cave_forward_backward_warm(_ex) with the pack's warm-start state when it has one, or
+    cave_forward_backward_resident when the pack also has a Gram cache."""
+    if pack is not None and pack.gram is not None:
+        *head, stream = args
+        nwarm = pack.warm.numel() if pack.warm is not None else 0
+        ndense = pack.warm_dense.numel() if pack.warm_dense is not None else 0
+        _lib.check(lib.cave_forward_backward_resident(*head, _ptr(pack.warm), nwarm, _ptr(pack.warm_dense), ndense,
+                                                      _ptr(pack.gram), pack.gram.numel(), stream))
+    elif pack is not None and pack.warm_dense is not None:
         *head, stream = args
         nwarm = pack.warm.numel() if pack.warm is not None else 0
         _lib.check(lib.cave_forward_backward_warm_ex(*head, _ptr(pack.warm), nwarm, _ptr(pack.warm_dense),

@@ -228,6 +228,45 @@ int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const v
                                   void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
                                   void* stream);
 
+/* Gram cache of a resident dense dataset: G~ = A A^T of every pack instance the dense path could take, computed once, so
+ * that later calls with the pack run neither the TF32 split nor the Gram kernel for their dense instances.  A caller-owned
+ * buffer over the N instances of a pack built by cave_pack():
+ *   [0]     int32 header: valid (1 once built), n_cached, m_pad (m_max rounded up to 128), N
+ *   [16]    int32 map[N]: the cache slot of pack instance q, or -1
+ *   [base]  base = (16 + 4 N) rounded up to 1024: n_cached slots of float32 [m_pad][m_pad], G~ of the instance's valid
+ *           rows in order, both triangles, zero outside the instance's leading square of 128-row blocks.
+ * An instance has a slot if it has no singleton row, >= 128 rows that are all general rows, and m_pad <= 2048: every
+ * instance that a call with any dense_mode puts on the dense path.
+ * cave_gram_cache_count(): the number of such instances of the pack into *n_cached_dev (device memory, on the stream).
+ * cave_gram_cache_bytes(): bytes of a cache for N instances with n_cached slots.
+ * cave_gram_cache_build(): fills the cache from A and its pack (cave_pack of the same A) with the same prep and Gram kernels
+ * a call runs; scratch must hold cave_scratch_bytes(N, ...) with dense_mode = 1 and the same opts (opts->dense_slots
+ * instances per round).  The buffer should be zeroed beforehand; it needs at least cave_gram_cache_bytes(N, 0, ...) bytes
+ * (CAVE_ENOSPC) and 16-byte alignment (CAVE_EINVAL); one that holds fewer than n_cached slots stays invalid.  Shapes
+ * outside the dense path: CAVE_ELIMIT (the count is then 0).
+ * cave_forward_backward_resident(): cave_forward_backward_warm_ex plus the cache.  Any of warm, warm_dense and gram may be
+ * null, not all three (CAVE_EINVAL); it needs opts->warm_pack = 1 (CAVE_EINVAL); gram needs A and 16-byte alignment
+ * (CAVE_EINVAL) and at least cave_gram_cache_bytes(pack instances, 0, ...) bytes (CAVE_ENOSPC).  Results are bit-identical to
+ * the same call without the cache.  A dense instance whose cache is not valid for this pack (header, m_pad, N or slot)
+ * reports CAVE_ST_BADINPUT | CAVE_ST_PATH_GRAM with NaN outputs.  Calls without the dense path (heuristic mode,
+ * dense_mode < 0, or a shape the host gate keeps off it) ignore the cache.  The cache is only read; it stays valid as long
+ * as A is not modified. */
+int cave_gram_cache_count(const void* pack, size_t pack_bytes, int64_t N, int64_t m_max, int64_t d, int32_t* n_cached_dev,
+                          void* stream);
+int cave_gram_cache_bytes(int64_t N, int64_t n_cached, int64_t m_max, int64_t d, size_t* out);
+int cave_gram_cache_build(const float* A, int64_t N, int64_t m_max, int64_t d, const cave_solver_opts* opts,
+                          void* cache, size_t cache_bytes, const void* pack, size_t pack_bytes,
+                          void* scratch, size_t scratch_bytes, void* stream);
+int cave_forward_backward_resident(const float* A, const int32_t* m_rows, const void* pred,
+                                   int64_t B, int64_t m_max, int64_t d,
+                                   double sign, int mode, double inner_ratio, int reduction,
+                                   int io_dtype, int compute_dtype, const cave_solver_opts* opts,
+                                   void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                   int32_t* status, int32_t* iters,
+                                   void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
+                                   void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                   const void* gram, size_t gram_bytes, void* stream);
+
 /* Diagnostic for the dense regime (north_star item 1): runs cave_pack() on A and then only the TF32 split and the
  * tensor-core Gram kernel (TMA tiles -> tcgen05.mma, 3xTF32, float32 accumulation in TMEM) for the first
  * min(B, slots) instances, and copies G~ = A A^T of instance i to G_out[i] as a row-major [m_pad, m_pad] float32
