@@ -294,16 +294,32 @@ __global__ void __launch_bounds__(NT) scan_kernel(ScanParams p) {
 }
 
 
+// one non-zero of a general row: its 2^-40 fixed-point share of the average, the int8 test and the two row hashes
+template <bool SKIPAVG>
+__device__ __forceinline__ void gen_elem(float v, int k, bool av, bool fits, float inv, unsigned long long* avg_fx, int* s_cnt,
+                                         uint64_t& hp, uint64_t& hn) {
+    if (av && !SKIPAVG) atomicAdd(&avg_fx[k], (unsigned long long)__double2ll_rn((double)v * (double)inv * 1099511627776.0));
+    if (fits) {
+        if (!(v == (float)(int)v && fabsf(v) <= 127.f)) s_cnt[7] = 1;      // not an int8 value
+        const uint32_t bits = __float_as_uint(v);
+        hp += mix64d(((uint64_t)k << 32) | bits);
+        hn += mix64d(((uint64_t)k << 32) | (bits ^ 0x80000000u));
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Warp-streaming variant (rows up to a few KB: every shipped model).  No CTA barrier in the steady
 // state: warp w owns rows w, w+8, ... of the instance and a private ring of row buffers that its lane 0
 // refills with TMA bulk copies, so eight independent row streams are in flight per CTA.  Cross-row
 // state is either warp-private (fixed order => reproducible) or exact under reordering (integer
 // atomics); the ordered general-row list is assembled once per instance after a single barrier.
+// Per row: one pass of 128-bit loads folded into one bit per non-zero word and one ballot; only the non-zero words are
+// read again.  92 % of the rows of a TSP-50 instance are singletons, so that slot is refilled as soon as the row is
+// classified; a general row refills after its CSR / hash pass, which visits the non-zero words only.
 // SKIPAVG: instantiation for packs that need no average (ScanParams::skip_avg); the default instantiation is textually the
 // round-1 kernel (a run-time test in the row loop changed its register allocation, 56 -> 48, and cost the TSP-50 scan 4 %).
 template <int NT, int S, bool SKIPAVG = false>
-__global__ void __launch_bounds__(NT) scan_rows_kernel(ScanParams p) {
+__global__ void __launch_bounds__(NT, 2) scan_rows_kernel(ScanParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     constexpr int NW = NT / 32;
@@ -366,43 +382,49 @@ __global__ void __launch_bounds__(NT) scan_rows_kernel(ScanParams p) {
         const float* base = (const float*)(myring + (size_t)s * rowbuf);
         mbar_wait(mybar + s, (uint32_t)((it / S) & 1));
 
+        // The row is split into units: lanes 0-3 each own one element of the ragged head (before the first whole 128-bit
+        // word) and one of the ragged tail, and lane L owns the whole words q0 + L + 32 j.  Pass 1 loads every unit and
+        // keeps one bit per non-zero unit (bit 0 head, bit 1 tail, bit 2 + j word j); one ballot then classifies the row.
+        // Only the non-zero units are visited again, in bit order, which is the per-lane order of the sums below.
         const int e0 = shift, e1 = e0 + d;
-        const int q0 = (e0 + 3) >> 2, q1 = e1 >> 2;
+        const int q0 = (e0 + 3) >> 2, q1 = e1 >> 2;         // [q0, q1): whole words; q0 > q1 only for d < 4 (head only)
+        const float4* b4 = (const float4*)base;
+        uint32_t nzw = 0;
+        if (lane < 4) {
+            const int kh = e0 + lane, kt = (q1 << 2) + lane;
+            if (kh < min(q0 << 2, e1) && (__float_as_uint(base[kh]) << 1) != 0u) nzw = 1u;      // (<< 1: -0.0 is a zero)
+            if (kt >= (q0 << 2) && kt < e1 && (__float_as_uint(base[kt]) << 1) != 0u) nzw |= 2u;
+        }
+        for (int q = q0 + lane, j = 2; q < q1 + lane; q += 128, j += 4) {     // uniform trip count; j < 20 (launch_scan: d < 2100)
+            uint32_t nib = 0;
+#pragma unroll
+            for (int u = 0; u < 4; ++u) {
+                if (q + 32 * u < q1) {
+                    const float4 v = b4[q + 32 * u];
+                    if (((__float_as_uint(v.x) | __float_as_uint(v.y) | __float_as_uint(v.z) | __float_as_uint(v.w)) << 1) != 0u)
+                        nib |= 1u << u;
+                }
+            }
+            nzw |= nib << j;
+        }
+        const unsigned sawm = __ballot_sync(0xffffffffu, nzw != 0u);
+        // exact non-zero count, |a|_1, |a|_2^2 and the last non-zero of every lane, in the lane's unit order
         RowAcc acc; acc.l1 = 0.f; acc.l2 = 0.f; acc.lv = 0.f; acc.lk = -1; acc.n = 0;
-        if (q0 <= q1) {
-            if (lane < 4) {
-                const int kh = e0 + lane;
-                if (kh < (q0 << 2) && kh < e1) { float v = base[kh]; if (v != 0.f) acc.add(v, kh - e0); }
-                const int kt = (q1 << 2) + lane;
-                if (kt >= (q0 << 2) && kt < e1) { float v = base[kt]; if (v != 0.f) acc.add(v, kt - e0); }
+        for (uint32_t m = nzw; m; m &= m - 1) {
+            const int bit = __ffs(m) - 1;
+            if (bit < 2) {
+                const int e = bit == 0 ? e0 + lane : (q1 << 2) + lane;
+                acc.add(base[e], e - e0);
+            } else {
+                const int q = q0 + lane + 32 * (bit - 2), k = (q << 2) - e0;
+                const float4 v = b4[q];
+                if (v.x != 0.f) acc.add(v.x, k);
+                if (v.y != 0.f) acc.add(v.y, k + 1);
+                if (v.z != 0.f) acc.add(v.z, k + 2);
+                if (v.w != 0.f) acc.add(v.w, k + 3);
             }
-            const float4* b4 = (const float4*)base;
-            for (int q = q0 + lane; q < q1 + lane; q += 128) {      // four independent 128-bit words per trip
-                float4 v[4];
-                uint32_t any[4];
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    v[u] = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (q + 32 * u < q1) v[u] = b4[q + 32 * u];
-                    any[u] = (__float_as_uint(v[u].x) | __float_as_uint(v[u].y) | __float_as_uint(v[u].z) | __float_as_uint(v[u].w)) << 1;
-                }
-                if (__ballot_sync(0xffffffffu, (any[0] | any[1] | any[2] | any[3]) != 0u) == 0u) continue;
-#pragma unroll
-                for (int u = 0; u < 4; ++u) {
-                    if (any[u] != 0u) {
-                        const int k = ((q + 32 * u) << 2) - e0;
-                        if (v[u].x != 0.f) acc.add(v[u].x, k);
-                        if (v[u].y != 0.f) acc.add(v[u].y, k + 1);
-                        if (v[u].z != 0.f) acc.add(v[u].z, k + 2);
-                        if (v[u].w != 0.f) acc.add(v[u].w, k + 3);
-                    }
-                }
-            }
-        } else {
-            for (int k = e0 + lane; k < e1; k += 32) { float v = base[k]; if (v != 0.f) acc.add(v, k - e0); }
         }
         int cnt = 0;
-        const unsigned sawm = __ballot_sync(0xffffffffu, acc.n > 0);
         if (sawm) {
             if ((sawm & (sawm - 1)) == 0u) {
                 cnt = __shfl_sync(0xffffffffu, acc.n, __ffs(sawm) - 1);
@@ -412,13 +434,21 @@ __global__ void __launch_bounds__(NT) scan_rows_kernel(ScanParams p) {
                 for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
             }
         }
+        if (cnt < 2) {
+            // an empty or singleton row is in registers now: its ring slot can take the next row before the bookkeeping
+            __syncwarp();
+            if (lane == 0 && it + S < nit) {
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                issue(it + S);
+            }
+        }
         if (cnt == 1) {
             const int src = __ffs(sawm) - 1;
-            const int k1 = __shfl_sync(0xffffffffu, acc.lk, src);
             const float v1 = __shfl_sync(0xffffffffu, acc.lv, src);
             const bool nv = fabsf(v1) > 1e-7f, av = sqrtf(v1 * v1) > 1e-7f;
             w_nvalid += nv; w_navg += av;
-            if (lane == 0) {
+            if (lane == src) {
+                const int k1 = acc.lk;
                 if (nv) atomicOr(&ctype_w[k1 >> 2], (v1 > 0.f ? 1u : 2u) << ((k1 & 3) * 8));
                 if (av) atomicAdd(&sing[k1], v1 > 0.f ? 1 : -1);
             }
@@ -443,27 +473,58 @@ __global__ void __launch_bounds__(NT) scan_rows_kernel(ScanParams p) {
                 w_gennnz += cnt; ++w_ngen;
                 w_l1max = fmaxf(w_l1max, a1); w_l2max = fmaxf(w_l2max, a2);
             }
-            uint64_t hp = 0, hn = 0;
-            const float* row = base + shift;
-            int w = off;
-            // (SKIPAVG: a row that does not fit the packed CSR has nothing left to do here: 1.25 M shared 64-bit atomics per
-            // 1024 x 1225 dense instance otherwise)
-            for (int k0 = 0; k0 < ((SKIPAVG && !fits) ? 0 : d); k0 += 32) {
-                const int k = k0 + lane;
-                const float v = k < d ? row[k] : 0.f;
-                const unsigned nzm = __ballot_sync(0xffffffffu, v != 0.f);
-                if (v != 0.f) {
-                    if (av && !SKIPAVG) atomicAdd(&avg_fx[k], (unsigned long long)__double2ll_rn((double)v * (double)inv * 1099511627776.0));
-                    if (fits) {
-                        const int pos = w + __popc(nzm & ((1u << lane) - 1u));
-                        col_out[pos] = (uint16_t)k; val_out[pos] = v;
-                        if (!(v == (float)(int)v && fabsf(v) <= 127.f)) s_cnt[7] = 1;      // not an int8 value
-                        const uint32_t bits = __float_as_uint(v);
-                        hp += mix64d(((uint64_t)k << 32) | bits);
-                        hn += mix64d(((uint64_t)k << 32) | (bits ^ 0x80000000u));
+            if (fits) {
+                // packed CSR in column order: head units, then the words by (j, lane), then tail units; a lane's position
+                // inside each group is the warp prefix of the non-zero counts (three ballots of the 0..4 count per word)
+                const unsigned lt = (1u << lane) - 1u;
+                const unsigned hm = __ballot_sync(0xffffffffu, nzw & 1u);
+                if (nzw & 1u) {
+                    const int pos = off + __popc(hm & lt);
+                    col_out[pos] = (uint16_t)lane; val_out[pos] = base[e0 + lane];
+                }
+                int w = off + __popc(hm);
+                for (uint32_t jm = __reduce_or_sync(0xffffffffu, nzw & ~3u); jm; jm &= jm - 1) {
+                    const int bit = __ffs(jm) - 1;
+                    const int q = q0 + lane + 32 * (bit - 2);
+                    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if ((nzw >> bit) & 1u) v = b4[q];
+                    const int n = (v.x != 0.f) + (v.y != 0.f) + (v.z != 0.f) + (v.w != 0.f);
+                    const unsigned c0 = __ballot_sync(0xffffffffu, n & 1), c1 = __ballot_sync(0xffffffffu, n & 2),
+                                   c2 = __ballot_sync(0xffffffffu, n & 4);
+                    int pos = w + __popc(c0 & lt) + 2 * __popc(c1 & lt) + 4 * __popc(c2 & lt);
+                    w += __popc(c0) + 2 * __popc(c1) + 4 * __popc(c2);
+                    if (n) {
+                        const int k = (q << 2) - e0;
+                        if (v.x != 0.f) { col_out[pos] = (uint16_t)k; val_out[pos++] = v.x; }
+                        if (v.y != 0.f) { col_out[pos] = (uint16_t)(k + 1); val_out[pos++] = v.y; }
+                        if (v.z != 0.f) { col_out[pos] = (uint16_t)(k + 2); val_out[pos++] = v.z; }
+                        if (v.w != 0.f) { col_out[pos] = (uint16_t)(k + 3); val_out[pos] = v.w; }
                     }
                 }
-                w += __popc(nzm);
+                const unsigned tm = __ballot_sync(0xffffffffu, nzw & 2u);
+                if (nzw & 2u) {
+                    const int e = (q1 << 2) + lane;
+                    const int pos = w + __popc(tm & lt);
+                    col_out[pos] = (uint16_t)(e - e0); val_out[pos] = base[e];
+                }
+            }
+            // average, int8 test and hashes: order-free, so every lane walks its own non-zero units
+            // (SKIPAVG: a row that does not fit the packed CSR has nothing left to do here: 1.25 M shared 64-bit atomics per
+            // 1024 x 1225 dense instance otherwise)
+            uint64_t hp = 0, hn = 0;
+            for (uint32_t m = (SKIPAVG && !fits) ? 0u : nzw; m; m &= m - 1) {
+                const int bit = __ffs(m) - 1;
+                if (bit < 2) {
+                    const int e = bit == 0 ? e0 + lane : (q1 << 2) + lane;
+                    gen_elem<SKIPAVG>(base[e], e - e0, av, fits, inv, avg_fx, s_cnt, hp, hn);
+                } else {
+                    const int q = q0 + lane + 32 * (bit - 2), k = (q << 2) - e0;
+                    const float4 v = b4[q];
+                    if (v.x != 0.f) gen_elem<SKIPAVG>(v.x, k, av, fits, inv, avg_fx, s_cnt, hp, hn);
+                    if (v.y != 0.f) gen_elem<SKIPAVG>(v.y, k + 1, av, fits, inv, avg_fx, s_cnt, hp, hn);
+                    if (v.z != 0.f) gen_elem<SKIPAVG>(v.z, k + 2, av, fits, inv, avg_fx, s_cnt, hp, hn);
+                    if (v.w != 0.f) gen_elem<SKIPAVG>(v.w, k + 3, av, fits, inv, avg_fx, s_cnt, hp, hn);
+                }
             }
             if (nv) {
 #pragma unroll
@@ -476,11 +537,11 @@ __global__ void __launch_bounds__(NT) scan_rows_kernel(ScanParams p) {
                     hash_out[row_id] = make_ulonglong2(hp, hn);
                 }
             }
-        }
-        __syncwarp();
-        if (lane == 0 && it + S < nit) {
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            issue(it + S);
+            __syncwarp();       // a general row reads its slot until here
+            if (lane == 0 && it + S < nit) {
+                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+                issue(it + S);
+            }
         }
     }
 
