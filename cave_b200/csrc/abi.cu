@@ -57,6 +57,18 @@ int sm_count() {                    // of the CURRENT device (cached per device:
     return 148;                     // B200; used only for sizing when no device is visible
 }
 
+// dynamic shared memory of the wide solve configuration on the current device (cached per device, as sm_count)
+cudaError_t wide_smem(int* out) {
+    static int cached[64] = {0};
+    int dev = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e != cudaSuccess) return e;
+    if (dev >= 0 && dev < 64 && cached[dev] > 0) { *out = cached[dev]; return cudaSuccess; }
+    e = cave::solve_wide_smem_bytes(out);
+    if (e == cudaSuccess && dev >= 0 && dev < 64) cached[dev] = *out;
+    return e;
+}
+
 bool solve_forced() {     // experiments: a single launch with explicit thread / CTA / shared-memory settings
     return getenv("CAVE_SOLVE_THREADS") || getenv("CAVE_SOLVE_CTAS_PER_SM") || getenv("CAVE_SOLVE_SMEM");
 }
@@ -192,7 +204,7 @@ int cave_plan_choice(const uint64_t* plan_host, int64_t d, int io_dtype, int com
     const cave::SolveConfig cfg = cave::solve_config(c);
     if (threads) *threads = cfg.threads;
     if (ctas_per_sm) *ctas_per_sm = cfg.ctas_per_sm;
-    if (smem_bytes) *smem_bytes = cfg.smem_bytes;
+    if (smem_bytes) *smem_bytes = c == cave::kWideConfig ? (int)pl[cave::PLAN_WIDE] : cfg.smem_bytes;
     return c;
 }
 
@@ -246,6 +258,10 @@ static int pack_impl(const float* A, const int32_t* m_rows, int64_t B, int64_t m
     // the cached solver setup pays off when the pack is reused (warm / dataset packs: cave_pack); a pack that lives for one
     // call (cold cave_forward_backward) keeps the in-solver setup: the setup kernel would cost what it saves
     pp.setup = emit_setup ? base + L.setup : nullptr; pp.setup_stride = L.setup_stride; pp.setup_cap_v = L.setup_cap_v;
+    if (cave::wide_config_enabled(m_max, d)) {
+        e = wide_smem(&pp.wide_smem);
+        if (e != cudaSuccess) return fail(CAVE_ECUDA, "solve kernel attributes: %s", cudaGetErrorString(e));
+    }
     if (!emit_setup) {
         // no cached setup in this pack: the valid word of every instance's setup block must say so (the pack buffer is the
         // caller's uninitialised memory, possibly a recycled pack)
@@ -429,15 +445,22 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         if (ce != cudaSuccess) return fail(CAVE_ECUDA, "solve kernel launch failed: %s", cudaGetErrorString(ce));
     } else {
         // every candidate configuration is enqueued; the pack's plan statistics select exactly one on the device
-        // and the others return immediately (no host round trip, a few microseconds of launch overhead)
+        // and the others return immediately (no host round trip, a few microseconds of launch overhead).  The wide
+        // configuration is a candidate for the shapes wide_config_enabled admits (the plan kernel recorded the same test).
         const int only = env_int("CAVE_SOLVE_CFG", -1);
+        const bool forced = only >= 0 && only < cave::kNumSolveConfigs;
         for (int i = 0; i < cave::kNumSolveConfigs; ++i) {
             const cave::SolveConfig cfg = cave::solve_config(i);
-            if (only >= 0 && only < cave::kNumSolveConfigs && i != only) continue;
+            if (forced && i != only) continue;
+            if (i == cave::kWideConfig && !forced && !cave::wide_config_enabled(m_max, d)) continue;
             int64_t grid = (int64_t)sm_count() * cfg.ctas_per_sm;
             if (grid > n_slots) grid = n_slots;
             sp.smem_bytes = cfg.smem_bytes;
-            sp.cfg_id = (only >= 0 && only < cave::kNumSolveConfigs) ? -1 : i;
+            if (i == cave::kWideConfig) {
+                ce = wide_smem(&sp.smem_bytes);
+                if (ce != cudaSuccess) return fail(CAVE_ECUDA, "solve kernel attributes: %s", cudaGetErrorString(ce));
+            }
+            sp.cfg_id = forced ? -1 : i;
             ce = cave::launch_solve(sp, compute_dtype == CAVE_F32, io_dtype == CAVE_F32, (int)grid, cfg.threads, st);
             g_launches += 1;
             if (ce != cudaSuccess) return fail(CAVE_ECUDA, "solve kernel launch failed: %s", cudaGetErrorString(ce));

@@ -119,17 +119,28 @@ CAVE_HD PackLayout make_pack_layout(int64_t B, int64_t m_max, int64_t d) {
 // The solver is latency bound, so small instances want many small CTAs per SM and large ones few big CTAs.
 // Which one applies depends on the data (general rows, +- pairs, non-zeros), which only the device knows
 // after the scan; the plan kernel therefore reduces per-instance shared-memory footprints into PlanStats and
-// every candidate configuration is launched — the ones the statistics do not select exit at once.
+// every candidate configuration is launched — the ones the statistics do not select exit at once.  The wide
+// configuration (one CTA per SM) is a candidate only for the shapes wide_config_enabled admits.
 enum { PLAN_N = 0, PLAN_SUM8 = 1, PLAN_SUM4 = 2, PLAN_MAXHOT8 = 3, PLAN_MAXHOT4 = 4,   // indices into plan[]
+       PLAN_WIDE = 5,       // dynamic shared memory of the one-CTA-per-SM configuration if the shape enqueues it, else 0
        PLAN_NO_AVG = 7 };   // != 0: the pack was written without the average unit normal (one-shot pack of an exact-mode call)
 constexpr int kOrderMaxBatch = 16384;     // beyond this the drain is negligible and instances are taken in index order
 struct SolveConfig { int threads, ctas_per_sm, smem_bytes; };
-constexpr int kNumSolveConfigs = 4;
+constexpr int kNumSolveConfigs = 5;
+constexpr int kWideConfig = 4;            // 256 threads x 1 CTA/SM
 CAVE_HD SolveConfig solve_config(int i) {
-    // 4 x 128 x 128 registers fills the register file; shared memory per CTA leaves room for the static part
-    const SolveConfig t[kNumSolveConfigs] = {{64, 8, 27520}, {128, 4, 56320}, {160, 3, 75776}, {256, 2, 112640}};
+    // 4 x 128 x 128 registers fills the register file; shared memory per CTA leaves room for the static part.  The wide
+    // configuration gets what one CTA may have, the per-block maximum less the kernel's static shared memory: a property of
+    // the device and of the compiled kernel, read at run time (solve_wide_smem_bytes, plan[PLAN_WIDE]), hence 0 here.
+    const SolveConfig t[kNumSolveConfigs] = {{64, 8, 27520}, {128, 4, 56320}, {160, 3, 75776}, {256, 2, 112640}, {256, 1, 0}};
     return t[i];
 }
+// Whether a shape enqueues the wide configuration (the ABI's launch loop, the plan kernel's PLAN_WIDE word and, through that
+// word, the device rule and cave_plan_choice all follow this one function).  m_max > d is the structured regime: a bound row
+// per variable (the dense path's gate relies on the same test).  d > 2048: every shipped model up to TSP-50 (d = 1225) and
+// VRP-20 fits its largest hot set into 256 x 2 and keeps exactly the launches it had; from TSP-80 (d = 3160) on the hot set
+// of a Newton solve (the Hessian of ~d/50 variables and its factor) outgrows the 110 KiB of that configuration.
+CAVE_HD bool wide_config_enabled(int64_t m_max, int64_t d) { return m_max > d && d > 2048; }
 CAVE_HD size_t a16(size_t v) { return (v + 15) & ~(size_t)15; }
 // Shared-memory footprint of one instance (bytes), mirroring the Arena requests of solver_core.cuh.
 //   hot  : arrays that must be in shared memory for the fast layout
@@ -151,17 +162,20 @@ CAVE_HD void instance_footprint(int64_t d, int64_t ngen, int64_t nv, int64_t nnz
     *hot = h; *work = w;
 }
 // Smallest configuration whose shared memory holds the average working set with 5 % to spare and the largest
-// hot set outright; the widest one otherwise.  io_extra: bytes added when c is stored in float64.
+// hot set outright; 256 x 2 otherwise, unless the largest hot set does not fit there but fits the wide configuration
+// and the shape enqueued it (plan[PLAN_WIDE] != 0).  io_extra: bytes added when c is stored in float64.
 CAVE_HD int choose_solve_config(const unsigned long long* plan, size_t th, size_t io_extra) {
     const unsigned long long n = plan[PLAN_N];
-    if (n == 0) return kNumSolveConfigs - 1;
+    if (n == 0) return kWideConfig - 1;
     const size_t avg = (size_t)((th == 8 ? plan[PLAN_SUM8] : plan[PLAN_SUM4]) / n) + io_extra;
     const size_t mx = (size_t)(th == 8 ? plan[PLAN_MAXHOT8] : plan[PLAN_MAXHOT4]) + io_extra;
-    for (int i = 0; i < kNumSolveConfigs - 1; ++i) {
+    for (int i = 0; i < kWideConfig - 1; ++i) {
         const size_t cap = (size_t)solve_config(i).smem_bytes;
         if (avg * 20 <= cap * 19 && mx + 1024 <= cap) return i;
     }
-    return kNumSolveConfigs - 1;
+    const size_t wide = (size_t)plan[PLAN_WIDE];
+    if (wide != 0 && mx + 1024 > (size_t)solve_config(kWideConfig - 1).smem_bytes && mx + 1024 <= wide) return kWideConfig;
+    return kWideConfig - 1;
 }
 
 // Solver scratch: [work counter + large-slot locks][loss64 B][rnorm64 B][status B][iters B][one small slot per CTA]

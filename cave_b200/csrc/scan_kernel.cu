@@ -859,6 +859,7 @@ __global__ void __launch_bounds__(256) plan_kernel(PlanParams p) {
     __shared__ unsigned long long hp[8][kPlanMaxRows];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int b = blockIdx.x * 8 + w;
+    if (b == 0 && lane == 0) p.plan[PLAN_WIDE] = wide_config_enabled(p.m_max, p.d) ? (unsigned long long)p.wide_smem : 0ull;
     if (b >= p.B) return;
     const int ngen = p.ngen[b], nnz = p.gennnz[b], ok = p.csr_ok[b];
     const bool dense_path = p.nsingc[b] == 0;

@@ -42,6 +42,7 @@ struct PlanParams {
     // setup kernel (cached per-instance solver setup, layout.cuh SetupBlock)
     const uint16_t* csr_col; const float* csr_val; int64_t cap_nnz;
     char* setup; int64_t setup_stride, setup_cap_v;
+    int wide_smem;              // dynamic shared memory of the wide solve configuration (solve_wide_smem_bytes)
 };
 cudaError_t launch_plan(const PlanParams& p, cudaStream_t stream);
 cudaError_t launch_clear_setup(char* setup, long long stride, int B, cudaStream_t stream);

@@ -2,4 +2,5 @@
 #include "solve_kernel_impl.cuh"
 namespace cave {
 template cudaError_t launch_solve_t<double, float>(const SolveParams&, int, int, cudaStream_t);
+template cudaError_t solve_static_smem_t<double, float>(size_t*);
 }

@@ -43,6 +43,29 @@ extern template cudaError_t launch_solve_t<float, double>(const SolveParams&, in
 extern template cudaError_t launch_solve_t<double, float>(const SolveParams&, int, int, cudaStream_t);
 extern template cudaError_t launch_solve_t<double, double>(const SolveParams&, int, int, cudaStream_t);
 
+template <class T, class TIO>
+cudaError_t solve_static_smem_t(size_t* out);                                                   // solve_inst_*.cu
+extern template cudaError_t solve_static_smem_t<float, float>(size_t*);
+extern template cudaError_t solve_static_smem_t<float, double>(size_t*);
+extern template cudaError_t solve_static_smem_t<double, float>(size_t*);
+extern template cudaError_t solve_static_smem_t<double, double>(size_t*);
+
+cudaError_t solve_wide_smem_bytes(int* out) {
+    int dev = 0, optin = 0;
+    cudaError_t e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    size_t st = 0, s[4] = {0, 0, 0, 0};
+    if (e == cudaSuccess) e = solve_static_smem_t<float, float>(&s[0]);
+    if (e == cudaSuccess) e = solve_static_smem_t<float, double>(&s[1]);
+    if (e == cudaSuccess) e = solve_static_smem_t<double, float>(&s[2]);
+    if (e == cudaSuccess) e = solve_static_smem_t<double, double>(&s[3]);
+    if (e != cudaSuccess) return e;
+    for (size_t v : s) st = v > st ? v : st;
+    // one figure for every instantiation: the pack's plan records it before the call's precision is known
+    *out = (int)(((size_t)optin - st) & ~(size_t)15);
+    return cudaSuccess;
+}
+
 cudaError_t launch_solve(const SolveParams& p, int compute_f32, int io_f32, int grid, int threads, cudaStream_t stream) {
     if (compute_f32) return io_f32 ? launch_solve_t<float, float>(p, grid, threads, stream)
                                    : launch_solve_t<float, double>(p, grid, threads, stream);

@@ -59,6 +59,9 @@ struct FinalizeParams {
 };
 
 cudaError_t launch_solve(const SolveParams& p, int compute_f32, int io_f32, int grid, int threads, cudaStream_t stream);
+// dynamic shared memory of the wide configuration (layout.cuh kWideConfig) on the current device: the per-block maximum less
+// the largest static shared memory of the solve kernels, rounded down to 16 bytes
+cudaError_t solve_wide_smem_bytes(int* out);
 cudaError_t launch_finalize(const FinalizeParams& p, int io_f32, cudaStream_t stream);
 
 }  // namespace cave

@@ -111,4 +111,15 @@ cudaError_t launch_solve_t(const SolveParams& p, int grid, int threads, cudaStre
     return p.warm ? launch_solve_v<T, TIO, true>(p, grid, threads, stream) : launch_solve_v<T, TIO, false>(p, grid, threads, stream);
 }
 
+// static shared memory of the two kernels of this (factor, I/O) pair, the larger one (the wide configuration's dynamic shared
+// memory is the per-block maximum less this)
+template <class T, class TIO>
+cudaError_t solve_static_smem_t(size_t* out) {
+    cudaFuncAttributes a, w;
+    cudaError_t e = cudaFuncGetAttributes(&a, solve_kernel<T, TIO, false>);
+    if (e == cudaSuccess) e = cudaFuncGetAttributes(&w, solve_kernel<T, TIO, true>);
+    if (e == cudaSuccess) *out = a.sharedSizeBytes > w.sharedSizeBytes ? a.sharedSizeBytes : w.sharedSizeBytes;
+    return e;
+}
+
 }  // namespace cave

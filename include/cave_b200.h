@@ -115,7 +115,10 @@ int cave_pack_bytes(int64_t B, int64_t m_max, int64_t d, size_t* out);
  * instances' shared-memory footprints into 8 uint64 statistics stored in the pack at cave_plan_offset(); the solve
  * kernel is enqueued in every candidate configuration and the statistics select one ON THE DEVICE (no host
  * round trip).  cave_plan_choice() applies the same rule to a host copy of those 8 words and returns the index
- * of the configuration that runs (threads per CTA, CTAs per SM, dynamic shared memory per CTA). */
+ * of the configuration that runs (threads per CTA, CTAs per SM, dynamic shared memory per CTA).  Word 5 is the dynamic
+ * shared memory of configuration 4 (256 threads, one CTA per SM) when the pack's shape enqueues it (structured
+ * instances with d > 2048), 0 otherwise; configuration 4 is chosen only when the largest hot set fits it but not
+ * configuration 3. */
 int cave_plan_offset(int64_t B, int64_t m_max, int64_t d, size_t* out);
 int cave_plan_choice(const uint64_t* plan_host, int64_t d, int io_dtype, int compute_dtype,
                      int* threads, int* ctas_per_sm, int* smem_bytes);
