@@ -84,25 +84,41 @@ def lawson_hanson(E: np.ndarray, f: np.ndarray, max_iter: int | None = None, tol
     return x, float(np.linalg.norm(E @ x - f))
 
 
-def project_nnls(cp: np.ndarray, ctr: np.ndarray, fp64_out: bool = False, use_scipy: bool = True):
+def is_projection(c: np.ndarray, ctr: np.ndarray, p: np.ndarray, tol: float = 1e-9) -> bool:
+    """Optimality conditions of p = lam @ ctr (lam >= 0) as the projection of c onto cone(ctr), in float64:
+    q = c - p lies in the polar cone (ctr q <= tol ||c|| max ||a_i||) and is orthogonal to p (|<p, q>| <= tol ||c||^2)."""
+    c, ctr, p = (np.asarray(x, np.float64) for x in (c, ctr, p))
+    q = c - p
+    cn = float(np.linalg.norm(c))
+    an = float(np.linalg.norm(ctr, axis=1).max(initial=0.0))
+    return float((ctr @ q).max(initial=0.0)) <= tol * cn * an and abs(float(p @ q)) <= tol * cn * cn
+
+
+def project_nnls(cp: np.ndarray, ctr: np.ndarray, fp64_out: bool = False, use_scipy: bool = True, certify: bool = False):
     """src/cave.py:298-309 `_project_nnls`: drop zero rows (303); empty -> (cp, 0.0) (304-305);
     nnls(ctr.T, cp) (306-307); p = lam @ ctr, cast float32 (308-309).
-    fp64_out=True returns the float64 projection *before* the float32 cast."""
+    fp64_out=True returns the float64 projection *before* the float32 cast.
+    certify=True: a SciPy result that fails `is_projection` is replaced by `lawson_hanson`'s, which must pass it (the
+    installed SciPy's nnls can stop at a non-optimal point on degenerate cones, e.g. rows a, a, -a, -a)."""
     ctr = ctr[np.abs(ctr).sum(axis=1) > ROW_TOL]
     if len(ctr) == 0:
         return (cp.astype(np.float64) if fp64_out else cp.astype(np.float32)), 0.0
     if use_scipy and _scipy_nnls is not None:
         lam, rnorm = _scipy_nnls(np.asfortranarray(ctr.T), cp)
+        if certify and not is_projection(cp, ctr, lam @ ctr):
+            lam, rnorm = lawson_hanson(ctr.T, cp)
+            if not is_projection(cp, ctr, lam @ ctr):
+                raise RuntimeError("neither nnls nor lawson_hanson meets the optimality conditions")
     else:
         lam, rnorm = lawson_hanson(ctr.T, cp)
     p = lam @ ctr
     return (np.asarray(p, dtype=np.float64) if fp64_out else p.astype(np.float32)), float(rnorm)
 
 
-def batch_project(signed_cost: np.ndarray, tight_ctrs: np.ndarray, fp64: bool = False):
+def batch_project(signed_cost: np.ndarray, tight_ctrs: np.ndarray, fp64: bool = False, certify: bool = False):
     """src/cave.py:231-264 `_batch_project`, solver='nnls', processes=1 (line 257):
-    stack per-instance results; rnorm goes through float32 (line 261) unless fp64."""
-    res = [project_nnls(signed_cost[i], tight_ctrs[i], fp64_out=fp64) for i in range(len(signed_cost))]
+    stack per-instance results; rnorm goes through float32 (line 261) unless fp64.  certify: see project_nnls."""
+    res = [project_nnls(signed_cost[i], tight_ctrs[i], fp64_out=fp64, certify=certify) for i in range(len(signed_cost))]
     proj = np.stack([r[0] for r in res])
     rnorm = np.asarray([r[1] for r in res], dtype=np.float64 if fp64 else np.float32)
     dt = np.float64 if fp64 else signed_cost.dtype
@@ -124,9 +140,9 @@ def _normalise(v: np.ndarray) -> np.ndarray:
     return v / np.maximum(np.linalg.norm(v, axis=1, keepdims=True), 1e-8)
 
 
-def exact_target(signed_cost, tight_ctrs, fp64=False):
+def exact_target(signed_cost, tight_ctrs, fp64=False, certify=False):
     """src/cave.py:121-129: proj / ||proj||.clamp(1e-8)."""
-    proj, rnorm = batch_project(signed_cost, tight_ctrs, fp64)
+    proj, rnorm = batch_project(signed_cost, tight_ctrs, fp64, certify)
     return _normalise(proj), proj, rnorm
 
 
@@ -136,9 +152,9 @@ def heuristic_target(signed_cost, tight_ctrs, inner_ratio):
     return (1 - inner_ratio) * _normalise(signed_cost) + inner_ratio * avg
 
 
-def inner_target(signed_cost, tight_ctrs, inner_ratio, fp64=False):
+def inner_target(signed_cost, tight_ctrs, inner_ratio, fp64=False, certify=False):
     """src/cave.py:206-219, solver='nnls' branch: where(rnorm < 1e-7, proj_norm, (1-r) proj_norm + r avg)."""
-    proj, rnorm = batch_project(signed_cost, tight_ctrs, fp64)
+    proj, rnorm = batch_project(signed_cost, tight_ctrs, fp64, certify)
     proj_norm = _normalise(proj)
     avg = average_ctrs(tight_ctrs).astype(proj.dtype)
     pushed = (1 - inner_ratio) * proj_norm + inner_ratio * avg
@@ -165,13 +181,14 @@ def cosine_loss_and_grad(c: np.ndarray, t: np.ndarray):
 
 def forward_backward(pred_cost: np.ndarray, tight_ctrs: np.ndarray, minimize: bool = True,
                      mode: int = MODE_EXACT, inner_ratio: float = 0.2, reduction: str = "mean",
-                     fp64: bool = False):
+                     fp64: bool = False, certify: bool = False):
     """src/cave.py:55-73 `forward` + autograd backward of the reduced loss w.r.t. pred_cost.
 
     mode: MODE_EXACT (exactConeAlignedCosine), MODE_INNER (innerConeAlignedCosine QP branch,
     solver='nnls'), MODE_HEURISTIC (innerConeAlignedCosine heuristic branch, src/cave.py:201-204).
     fp64=True: all arithmetic in float64 without the reference's float32 casts (parity target for
     the CUDA path's fp64 mode); fp64=False: follows the reference's dtypes (float32 in / out).
+    certify=True: every projection meets its optimality conditions (see project_nnls).
     Returns dict(loss, loss_i, grad, proj, rnorm, target)."""
     dt = np.float64 if fp64 else pred_cost.dtype
     pred = pred_cost.astype(dt)
@@ -182,9 +199,9 @@ def forward_backward(pred_cost: np.ndarray, tight_ctrs: np.ndarray, minimize: bo
     if mode == MODE_HEURISTIC:
         t = heuristic_target(c, ctrs, inner_ratio)
     elif mode == MODE_INNER:
-        t, proj, rnorm = inner_target(c, ctrs, inner_ratio, fp64)
+        t, proj, rnorm = inner_target(c, ctrs, inner_ratio, fp64, certify)
     else:
-        t, proj, rnorm = exact_target(c, ctrs, fp64)
+        t, proj, rnorm = exact_target(c, ctrs, fp64, certify)
     t = t.astype(dt)
     loss_i, grad_c = cosine_loss_and_grad(c, t)
     B = len(pred)

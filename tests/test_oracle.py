@@ -107,3 +107,18 @@ def test_analytic_gradient_matches_autograd():
     lt.sum().backward()
     np.testing.assert_allclose(loss, lt.detach().numpy(), rtol=1e-12, atol=1e-14)
     np.testing.assert_allclose(grad, ct.grad.numpy(), rtol=1e-9, atol=1e-12)
+
+
+def test_certified_projection_meets_the_optimality_conditions_on_degenerate_cones():
+    """certify=True: on cones with duplicated and opposite rows (tests/adversarial.py pm_pairs) every projection meets
+    is_projection and equals the independent Lawson-Hanson restatement, whatever scipy's nnls returned."""
+    import adversarial as adv
+    A, pred, _ = adv.batch("pm_pairs")
+    for b in range(0, len(A), 3):
+        a = A[b][np.abs(A[b]).sum(axis=1) > 0].astype(np.float64)
+        c = -pred[b].astype(np.float64)
+        p, r = O.project_nnls(c, a, fp64_out=True, certify=True)
+        assert O.is_projection(c, a, p)
+        lam, r_lh = O.lawson_hanson(a.T, c)
+        np.testing.assert_allclose(p, lam @ a, rtol=1e-9, atol=1e-10 * np.linalg.norm(c))
+        np.testing.assert_allclose(r, r_lh, rtol=1e-9, atol=1e-12)
