@@ -21,7 +21,8 @@ EXPORTS = ("cave_abi_version", "cave_last_error", "cave_get_limits", "cave_pack_
            "cave_dense_gram", "cave_launch_count", "cave_dense_ctrl_offset", "cave_pack_sparse",
            "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm",
            "cave_dense_warm_bytes", "cave_forward_backward_warm_ex", "cave_gram_cache_count", "cave_gram_cache_bytes",
-           "cave_gram_cache_build", "cave_forward_backward_resident")
+           "cave_gram_cache_build", "cave_forward_backward_resident", "cave_chunk_acc_bytes", "cave_forward_backward_chunk",
+           "cave_chunk_finalize", "cave_csr_rebase")
 
 
 class SolverOpts(ctypes.Structure):
@@ -76,6 +77,13 @@ def load() -> ctypes.CDLL:
                                                    ctypes.POINTER(SolverOpts), P, P, P, P, P, P, P,
                                                    P, ctypes.c_size_t, P, ctypes.c_size_t, P, ctypes.c_size_t,
                                                    P, ctypes.c_size_t, P, ctypes.c_size_t, P]
+    lib.cave_chunk_acc_bytes.argtypes = [I64, SZP]
+    lib.cave_forward_backward_chunk.argtypes = [P, P, P, I64, I64, I64, F, I32, F, I32, I32, I32,
+                                                ctypes.POINTER(SolverOpts), P, P, P, P, P, P, P,
+                                                P, ctypes.c_size_t, P, ctypes.c_size_t, P, ctypes.c_size_t,
+                                                P, ctypes.c_size_t, P, ctypes.c_size_t, I64, I64, P, ctypes.c_size_t, P]
+    lib.cave_chunk_finalize.argtypes = [P, ctypes.c_size_t, I64, I32, I32, P, P, P, P, P, P]
+    lib.cave_csr_rebase.argtypes = [P, I64, I64, P, I64, I64, P]
     lib.cave_gram_cache_count.argtypes = [P, ctypes.c_size_t, I64, I64, I64, P, P]
     lib.cave_gram_cache_bytes.argtypes = [I64, I64, I64, I64, SZP]
     lib.cave_gram_cache_build.argtypes = [P, I64, I64, I64, ctypes.POINTER(SolverOpts), P, ctypes.c_size_t, P, ctypes.c_size_t,
@@ -94,7 +102,8 @@ def load() -> ctypes.CDLL:
                  "cave_plan_offset", "cave_plan_choice", "cave_dense_gram", "cave_dense_ctrl_offset", "cave_pack_sparse",
                  "cave_tsp_scratch_bytes", "cave_tsp_solve", "cave_pack_ex", "cave_warm_bytes", "cave_forward_backward_warm",
                  "cave_dense_warm_bytes", "cave_forward_backward_warm_ex", "cave_gram_cache_count", "cave_gram_cache_bytes",
-                 "cave_gram_cache_build", "cave_forward_backward_resident"):
+                 "cave_gram_cache_build", "cave_forward_backward_resident", "cave_chunk_acc_bytes", "cave_forward_backward_chunk",
+           "cave_chunk_finalize", "cave_csr_rebase"):
         getattr(lib, name).restype = I32
     _lib = lib
     return lib

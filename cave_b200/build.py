@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB = os.path.join(OUT_DIR, "libcave_b200.so")
 SOURCES = ["scan_kernel.cu", "solve_kernel.cu", "solve_inst_f32_f32.cu", "solve_inst_f32_f64.cu",
-           "solve_inst_f64_f32.cu", "solve_inst_f64_f64.cu", "gram_kernel.cu", "dense_solve.cu", "tsp_dp.cu", "abi.cu"]
+           "solve_inst_f64_f32.cu", "solve_inst_f64_f64.cu", "gram_kernel.cu", "dense_solve.cu", "tsp_dp.cu", "chunk.cu", "abi.cu"]
 HEADERS = ["ctx.cuh", "layout.cuh", "dense.cuh", "scan_kernel.cuh", "solve_kernel.cuh", "solve_kernel_impl.cuh", "solver_core.cuh",
            os.path.join("..", "..", "include", "cave_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",

@@ -25,7 +25,8 @@ from .qpsolver import CavePack, SparseConstraints, cave_forward_backward, projec
 _REFERENCE_SOLVERS = ("apgd", "clarabel", "nnls")
 # constructor-level solver_kwargs: properties of the solver, never of one particular batch (a pack, an index or a row-count
 # hint belongs to a call; accepted here they would silently apply to every later batch)
-_KERNEL_KWARGS = ("precision", "max_iter", "max_linesearch", "tol", "cap_rows", "cap_nnz", "device", "dense", "dense_slots", "strict")
+_KERNEL_KWARGS = ("precision", "max_iter", "max_linesearch", "tol", "cap_rows", "cap_nnz", "device", "dense", "dense_slots", "strict",
+                  "chunk")
 
 
 class _CaveCudaFunction(torch.autograd.Function):

@@ -18,6 +18,10 @@ namespace cave {       // tsp_dp.cu (auxiliary: exact TSP for regret evaluation)
 size_t tsp_slot_floats(int n);
 cudaError_t launch_tsp(const float* cost, int N, int n, int* tour, double* obj, void* scratch, int n_slots, cudaStream_t stream);
 }
+namespace cave {       // chunk.cu
+cudaError_t launch_csr_rebase(long long* inst_off, long long n_inst_off, long long row_base, long long* row_ptr,
+                              long long n_row_ptr, long long nnz_base, cudaStream_t stream);
+}
 
 namespace {
 
@@ -154,6 +158,30 @@ int64_t dense_slots(const cave_solver_opts* o, int64_t B, int64_t m_max, int64_t
         if (n < sms) n = sms;
     }
     return n < B ? n : B;
+}
+
+// whole-batch accumulator of a chunked call (cave_chunk_acc_bytes): per-instance float64 loss / rnorm, int32 status / iters
+struct AccLayout { size_t loss64, rnorm64, status, iters, total; };
+AccLayout acc_layout(int64_t B_total) {
+    AccLayout L;
+    size_t o = 0;
+    L.loss64 = o;  o = cave::align_up(o + (size_t)B_total * 8, 256);
+    L.rnorm64 = o; o = cave::align_up(o + (size_t)B_total * 8, 256);
+    L.status = o;  o = cave::align_up(o + (size_t)B_total * 4, 256);
+    L.iters = o;   o = cave::align_up(o + (size_t)B_total * 4, 256);
+    L.total = o;
+    return L;
+}
+
+int check_acc(const void* acc, size_t acc_bytes, int64_t batch_total) {
+    if (batch_total <= 0) return fail(CAVE_EINVAL, "batch_total must be positive (got %lld)", (long long)batch_total);
+    if (batch_total > kMaxB) return fail(CAVE_ELIMIT, "batch_total = %lld exceeds the supported maximum", (long long)batch_total);
+    if (!acc) return fail(CAVE_EINVAL, "acc must not be null");
+    if (((uintptr_t)acc & 255) != 0) return fail(CAVE_EINVAL, "acc must be 256-byte aligned");
+    const size_t need = acc_layout(batch_total).total;
+    if (acc_bytes < need) return fail(CAVE_ENOSPC, "accumulator has %zu bytes, %zu needed (cave_chunk_acc_bytes of %lld instances)",
+                                      acc_bytes, need, (long long)batch_total);
+    return CAVE_OK;
 }
 
 }  // namespace
@@ -307,15 +335,19 @@ int cave_dense_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t*
 }
 
 // cave_forward_backward and its warm-start variants: warm / warm_dense are null for the former, checked buffers (either
-// may be null) for the latter
+// may be null) for the latter.  Rows [batch_offset, batch_offset + B) of a batch of batch_total rows: the unchunked entries
+// pass (0, B, null), and the per-instance results then go to the scratch and are finalized here; a chunk (acc set, checked by
+// the caller) writes them to acc at batch_offset and leaves the finalize to cave_chunk_finalize
 static int forward_backward_impl(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
                                  double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
                                  const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
                                  int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
                                  size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense,
-                                 size_t warm_dense_bytes, const void* gram, size_t gram_bytes, void* stream) {
+                                 size_t warm_dense_bytes, const void* gram, size_t gram_bytes, int64_t batch_offset,
+                                 int64_t batch_total, void* acc, void* stream) {
     const bool indexed = opts && opts->inst_index;
-    if ((!A && !indexed) || !pred || !loss_i || !grad || !pack || !scratch) return fail(CAVE_EINVAL, "A, pred, loss_i, grad, pack, scratch must not be null");
+    if ((!A && !indexed) || !pred || (!loss_i && !acc) || !grad || !pack || !scratch)
+        return fail(CAVE_EINVAL, "A, pred, loss_i, grad, pack, scratch must not be null");
     if (indexed && !opts->warm_pack) return fail(CAVE_EINVAL, "inst_index needs warm_pack (a pack built over the whole dataset)");
     if (indexed && opts->n_packed <= 0) return fail(CAVE_EINVAL, "n_packed must be positive with inst_index");
     if (int e = check_shape(B, m_max, d)) return e;
@@ -325,7 +357,7 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         return fail(CAVE_EINVAL, "bad dtype (io %d, compute %d)", io_dtype, compute_dtype);
     if (!(sign == 1.0 || sign == -1.0)) return fail(CAVE_EINVAL, "sign must be +1 or -1");
     if (!(inner_ratio >= 0.0 && inner_ratio <= 1.0)) return fail(CAVE_EINVAL, "inner_ratio must be in [0, 1]");
-    if (reduction != CAVE_REDUCE_NONE && !loss) return fail(CAVE_EINVAL, "loss must not be null for mean/sum");
+    if (!acc && reduction != CAVE_REDUCE_NONE && !loss) return fail(CAVE_EINVAL, "loss must not be null for mean/sum");
     if (((uintptr_t)scratch & 255) != 0 || ((uintptr_t)pack & 255) != 0) return fail(CAVE_EINVAL, "pack and scratch must be 256-byte aligned");
 
     const int64_t Bpack = indexed ? opts->n_packed : B;
@@ -385,12 +417,20 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
     sp.csr_ok = (const int*)(pb + PL.csrok); sp.maxl1 = (const float*)(pb + PL.maxl1); sp.maxl2 = (const float*)(pb + PL.maxl2);
     sp.ghash = (const ulonglong2*)(pb + PL.ghash); sp.csr_col = (const uint16_t*)(pb + PL.csr_col);
     sp.csr_val = (const float*)(pb + PL.csr_val); sp.cap_nnz = PL.cap_nnz;
-    sp.counter = (int*)(sb + SL.counter); sp.loss64 = (double*)(sb + SL.loss64); sp.rnorm64 = (double*)(sb + SL.rnorm64);
-    sp.status = (int*)(sb + SL.status); sp.iters = (int*)(sb + SL.iters);
+    sp.counter = (int*)(sb + SL.counter);
+    if (acc) {
+        const AccLayout AL = acc_layout(batch_total);
+        char* ab = (char*)acc;
+        sp.loss64 = (double*)(ab + AL.loss64) + batch_offset; sp.rnorm64 = (double*)(ab + AL.rnorm64) + batch_offset;
+        sp.status = (int*)(ab + AL.status) + batch_offset; sp.iters = (int*)(ab + AL.iters) + batch_offset;
+    } else {
+        sp.loss64 = (double*)(sb + SL.loss64); sp.rnorm64 = (double*)(sb + SL.rnorm64);
+        sp.status = (int*)(sb + SL.status); sp.iters = (int*)(sb + SL.iters);
+    }
     sp.slots = sb + SL.slots; sp.slot_bytes = SL.slot_bytes;
     sp.large = sb + SL.large; sp.large_bytes = SL.large_bytes; sp.n_large = (int)SL.n_large;
     sp.mode = mode; sp.inner_ratio = inner_ratio; sp.sign = sign;
-    sp.gscale = reduction == CAVE_REDUCE_MEAN ? 1.0 / (double)B : 1.0;
+    sp.gscale = reduction == CAVE_REDUCE_MEAN ? 1.0 / (double)batch_total : 1.0;
     sp.max_iter = opts ? opts->max_iter : 0; sp.max_ls = opts ? opts->max_linesearch : 0; sp.tol = opts ? opts->tol : 0.0;
     sp.inst_index = indexed ? opts->inst_index : nullptr;
     sp.plan = (const unsigned long long*)(pb + PL.plan);
@@ -467,6 +507,7 @@ static int forward_backward_impl(const float* A, const int32_t* m_rows, const vo
         }
     }
 
+    if (acc) return CAVE_OK;
     cave::FinalizeParams fp;
     memset(&fp, 0, sizeof(fp));
     fp.B = (int)B; fp.reduction = reduction; fp.loss64 = sp.loss64; fp.rnorm64 = sp.rnorm64; fp.status = sp.status; fp.iters = sp.iters;
@@ -484,7 +525,7 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
                           size_t scratch_bytes, void* stream) {
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 nullptr, 0, nullptr, 0, nullptr, 0, stream);
+                                 nullptr, 0, nullptr, 0, nullptr, 0, 0, B, nullptr, stream);
 }
 
 int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -497,7 +538,7 @@ int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void
         return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, nullptr, 0, nullptr, 0, stream);
+                                 warm, warm_bytes, nullptr, 0, nullptr, 0, 0, B, nullptr, stream);
 }
 
 int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -512,7 +553,7 @@ int cave_forward_backward_warm_ex(const float* A, const int32_t* m_rows, const v
         return fail(CAVE_EINVAL, "warm-start state needs opts->warm_pack = 1: it belongs to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, warm_dense, warm_dense_bytes, nullptr, 0, stream);
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, nullptr, 0, 0, B, nullptr, stream);
 }
 
 int cave_forward_backward_resident(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
@@ -527,7 +568,68 @@ int cave_forward_backward_resident(const float* A, const int32_t* m_rows, const 
         return fail(CAVE_EINVAL, "warm-start state and Gram cache need opts->warm_pack = 1: they belong to a pack built beforehand by cave_pack()");
     return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
                                  loss, loss_i, grad, proj, rnorm, status, iters, pack, pack_bytes, scratch, scratch_bytes,
-                                 warm, warm_bytes, warm_dense, warm_dense_bytes, gram, gram_bytes, stream);
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, gram, gram_bytes, 0, B, nullptr, stream);
+}
+
+int cave_chunk_acc_bytes(int64_t B_total, size_t* out) {
+    if (!out) return fail(CAVE_EINVAL, "out is null");
+    if (B_total <= 0) return fail(CAVE_EINVAL, "B_total must be positive (got %lld)", (long long)B_total);
+    if (B_total > kMaxB) return fail(CAVE_ELIMIT, "B_total = %lld exceeds the supported maximum", (long long)B_total);
+    *out = acc_layout(B_total).total;
+    return CAVE_OK;
+}
+
+int cave_forward_backward_chunk(const float* A, const int32_t* m_rows, const void* pred, int64_t B, int64_t m_max, int64_t d,
+                                double sign, int mode, double inner_ratio, int reduction, int io_dtype, int compute_dtype,
+                                const cave_solver_opts* opts, void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                int32_t* status, int32_t* iters, void* pack, size_t pack_bytes, void* scratch,
+                                size_t scratch_bytes, void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                const void* gram, size_t gram_bytes, int64_t batch_offset, int64_t batch_total, void* acc,
+                                size_t acc_bytes, void* stream) {
+    if (int e = check_acc(acc, acc_bytes, batch_total)) return e;
+    if (batch_offset < 0 || batch_offset + B > batch_total)
+        return fail(CAVE_EINVAL, "chunk rows [%lld, %lld + %lld) are not inside the batch of %lld rows", (long long)batch_offset,
+                    (long long)batch_offset, (long long)B, (long long)batch_total);
+    if ((warm || warm_dense || gram) && !(opts && opts->warm_pack))
+        return fail(CAVE_EINVAL, "warm-start state and Gram cache need opts->warm_pack = 1: they belong to a pack built beforehand by cave_pack()");
+    (void)loss; (void)loss_i; (void)rnorm; (void)status; (void)iters;     // written by cave_chunk_finalize
+    return forward_backward_impl(A, m_rows, pred, B, m_max, d, sign, mode, inner_ratio, reduction, io_dtype, compute_dtype, opts,
+                                 nullptr, nullptr, grad, proj, nullptr, nullptr, nullptr, pack, pack_bytes, scratch, scratch_bytes,
+                                 warm, warm_bytes, warm_dense, warm_dense_bytes, gram, gram_bytes, batch_offset, batch_total, acc,
+                                 stream);
+}
+
+int cave_chunk_finalize(const void* acc, size_t acc_bytes, int64_t batch_total, int reduction, int io_dtype, void* loss,
+                        void* loss_i, void* rnorm, int32_t* status, int32_t* iters, void* stream) {
+    if (int e = check_acc(acc, acc_bytes, batch_total)) return e;
+    if (reduction < CAVE_REDUCE_MEAN || reduction > CAVE_REDUCE_NONE) return fail(CAVE_EINVAL, "bad reduction %d", reduction);
+    if (io_dtype != CAVE_F32 && io_dtype != CAVE_F64) return fail(CAVE_EINVAL, "bad io_dtype %d", io_dtype);
+    if (!loss_i) return fail(CAVE_EINVAL, "loss_i must not be null");
+    if (reduction != CAVE_REDUCE_NONE && !loss) return fail(CAVE_EINVAL, "loss must not be null for mean/sum");
+    const AccLayout AL = acc_layout(batch_total);
+    const char* ab = (const char*)acc;
+    cave::FinalizeParams fp;
+    memset(&fp, 0, sizeof(fp));
+    fp.B = (int)batch_total; fp.reduction = reduction;
+    fp.loss64 = (const double*)(ab + AL.loss64); fp.rnorm64 = (const double*)(ab + AL.rnorm64);
+    fp.status = (const int*)(ab + AL.status); fp.iters = (const int*)(ab + AL.iters);
+    fp.loss = loss; fp.loss_i = loss_i; fp.rnorm = rnorm; fp.status_out = status; fp.iters_out = iters;
+    cudaError_t ce = cave::launch_finalize(fp, io_dtype == CAVE_F32, (cudaStream_t)stream);
+    g_launches += 1;
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "finalize kernel launch failed: %s", cudaGetErrorString(ce));
+    return CAVE_OK;
+}
+
+int cave_csr_rebase(int64_t* inst_off, int64_t n_inst_off, int64_t row_base, int64_t* row_ptr, int64_t n_row_ptr,
+                    int64_t nnz_base, void* stream) {
+    if (n_inst_off < 0 || n_row_ptr < 0) return fail(CAVE_EINVAL, "array lengths must not be negative");
+    if ((n_inst_off && !inst_off) || (n_row_ptr && !row_ptr)) return fail(CAVE_EINVAL, "inst_off and row_ptr must not be null");
+    if (n_inst_off + n_row_ptr == 0) return CAVE_OK;
+    cudaError_t ce = cave::launch_csr_rebase((long long*)inst_off, n_inst_off, row_base, (long long*)row_ptr, n_row_ptr, nnz_base,
+                                             (cudaStream_t)stream);
+    g_launches += 1;
+    if (ce != cudaSuccess) return fail(CAVE_ECUDA, "CSR rebase kernel launch failed: %s", cudaGetErrorString(ce));
+    return CAVE_OK;
 }
 
 int cave_gram_cache_bytes(int64_t N, int64_t n_cached, int64_t m_max, int64_t d, size_t* out) {

@@ -14,6 +14,7 @@ hand-written sm_100a kernels behind the C ABI of include/cave_b200.h.  No CPU fa
 from __future__ import annotations
 
 import ctypes
+import numbers
 import os
 from dataclasses import dataclass
 
@@ -289,12 +290,24 @@ def cave_forward_backward(pred_cost: torch.Tensor, tight_ctrs: torch.Tensor, sig
                           want_proj: bool = False, want_status: bool = False, pack: CavePack | None = None,
                           index: torch.Tensor | None = None,
                           m_rows: torch.Tensor | None = None, device=None, max_iter=None, max_linesearch=None,
-                          tol=None, cap_rows=None, cap_nnz=None, dense="auto", dense_slots=None) -> dict:
+                          tol=None, cap_rows=None, cap_nnz=None, dense="auto", dense_slots=None, chunk=None) -> dict:
     """One call of the hot path through the C ABI.  Returns a dict with ``loss`` (scalar for
     mean/sum, [B] for none), ``loss_i`` [B], ``grad`` [B, d] (= d loss / d pred_cost for an upstream
     gradient of one), and optionally ``proj``, ``rnorm``, ``status``, ``iters`` — all on the
-    compute device, in ``pred_cost``'s dtype."""
+    compute device, in ``pred_cost``'s dtype.
+
+    ``chunk``: solve the batch ``chunk`` rows at a time, copying the next chunk's inputs to the device and the last chunk's
+    gradient back while a chunk is solved (``_forward_backward_chunked``).  Device memory then scales with ``chunk``, not
+    with the batch.  The results are those of the unchunked call (see there for the one-shot packs); ``None`` or
+    ``chunk >= B`` is the unchunked call."""
+    if chunk is not None and (isinstance(chunk, bool) or not isinstance(chunk, numbers.Integral) or chunk <= 0):
+        raise ValueError(f"chunk must be a positive int or None (got {chunk!r})")
     lib = _lib.load()
+    if chunk is not None and 0 < int(chunk) < pred_cost.shape[0]:
+        return _forward_backward_chunked(lib, pred_cost, tight_ctrs, sign, mode, inner_ratio, reduction, precision, want_proj,
+                                         want_status, pack, index, m_rows, device, int(chunk),
+                                         dict(max_iter=max_iter, max_linesearch=max_linesearch, tol=tol, cap_rows=cap_rows,
+                                              cap_nnz=cap_nnz, dense=dense, dense_slots=dense_slots))
     if isinstance(tight_ctrs, SparseConstraints):      # one-shot sparse batch: pack from the non-zeros, then the indexed path
         pack = pack_constraints_sparse(tight_ctrs, device=device, cache_setup=False)
         tight_ctrs = None
@@ -412,6 +425,258 @@ def _forward_backward_indexed(lib, pred_cost, ctrs, sign, mode, inner_ratio, red
         out["proj"], out["rnorm"] = proj, rnorm
     if want_status:
         out["status"], out["iters"], out["rnorm"] = status, iters, rnorm
+    return out
+
+
+def chunk_bounds(B: int, chunk: int) -> list[tuple[int, int]]:
+    """Rows ``[lo, hi)`` of the consecutive chunks of a batch of ``B`` rows (the last one may be shorter)."""
+    return [(lo, min(lo + chunk, B)) for lo in range(0, B, chunk)]
+
+
+class _Ring:
+    """Chunks of one host tensor on their way to the device: two device buffers that alternate between chunks, each sized for
+    the largest chunk, and for pageable memory two pinned buffers in front of them (a pinned source is copied directly)."""
+
+    def __init__(self, src: torch.Tensor, cap: int, dev: torch.device):
+        self.src = src
+        shape = (max(cap, 1),) + tuple(src.shape[1:])
+        self.dev = [torch.empty(shape, dtype=src.dtype, device=dev) for _ in range(2)]
+        self.pin = None if src.is_pinned() else [torch.empty(shape, dtype=src.dtype, pin_memory=True) for _ in range(2)]
+
+    def nbytes(self) -> int:
+        return sum(t.numel() * t.element_size() for t in self.dev)
+
+    def put(self, s: int, lo: int, hi: int, copied: torch.cuda.Event) -> torch.Tensor:
+        """Enqueues the copy of rows [lo, hi) into set ``s`` on the current (copy) stream; ``copied`` is the event recorded
+        after the previous copy out of set ``s`` (the host waits for it before it overwrites the pinned buffer)."""
+        n = hi - lo
+        src = self.src[lo:hi]
+        if self.pin is not None:
+            copied.synchronize()
+            self.pin[s][:n].copy_(src)
+            src = self.pin[s][:n]
+        dst = self.dev[s][:n]
+        dst.copy_(src, non_blocking=True)
+        return dst
+
+
+def _forward_backward_chunked(lib, pred_cost, ctrs, sign, mode, inner_ratio, reduction, precision, want_proj, want_status,
+                              pack, index, m_rows, device, chunk, solver) -> dict:
+    """``cave_forward_backward(..., chunk=chunk)`` for ``chunk < B``: the batch as consecutive chunks of ``chunk`` rows
+    (``cave_forward_backward_chunk``), then one ``cave_chunk_finalize`` over the whole batch.
+
+    Inputs: a dense ``[B, m, d]`` tensor (a one-shot pack per chunk), ``SparseConstraints`` (a one-shot sparse pack per
+    chunk) or a resident pack with ``index`` (or a pack of exactly ``ctrs``: slices of the index and the predictions only).
+    Host inputs are copied chunk by chunk on a side stream into two alternating device buffers (through two pinned buffers
+    when the host memory is pageable), the kernels of each chunk run on the caller's current stream, and with a host
+    ``pred_cost`` the gradient (and projection) of each chunk is copied on a second side stream into pinned host outputs; all
+    outputs are then host tensors and the call synchronises.  Device inputs are sliced in place.  Pack and scratch are
+    sized for one chunk.
+
+    Every instance is solved on its own, so the per-instance results are the unchunked call's, and the finalize reduces the
+    whole batch in the unchunked order.  A one-shot pack (dense or sparse input) selects the solve kernel's launch
+    configuration from its own instances, so a chunk can run another configuration than the whole batch: its results then
+    agree to rounding only (bit-identical with the configuration fixed, ``CAVE_SOLVE_CFG``).  A warm pack's slots are
+    written by a chunk before the next chunk reads them (one stream); an index that holds an instance in two chunks can
+    therefore start the second solve from the first one's solution."""
+    if reduction not in _lib.REDUCE:
+        raise ValueError(f"No reduction '{reduction}'.")
+    if precision not in _PRECISIONS:
+        raise ValueError(f"precision must be one of {sorted(_PRECISIONS)}")
+    sparse = isinstance(ctrs, SparseConstraints)
+    resident = pack is not None and not sparse
+    B = pred_cost.shape[0]
+    if pred_cost.dim() != 2:
+        raise ValueError(f"pred_cost must be [B, d], got {tuple(pred_cost.shape)}")
+    if resident:
+        dev = pack.buf.device
+        N, m, d = pack.shape
+        if index is None:
+            if ctrs is None and N != B:
+                raise ValueError("index= is needed unless the pack holds exactly the batch")
+            if ctrs is not None and (pack.data_ptr != ctrs.data_ptr() or pack.version != int(ctrs._version)):
+                raise ValueError("pack does not belong to this tight_ctrs tensor (other storage, or the tensor was modified "
+                                 "in place after pack_constraints)")
+            index = torch.arange(B, dtype=torch.int32, device=dev)
+        A = ctrs if ctrs is not None else pack.ctrs
+        if A is not None and (not A.is_cuda or A.device != dev or tuple(A.shape) != (N, m, d) or A.dtype != torch.float32):
+            raise ValueError("the dense dataset tensor must be the float32 CUDA tensor the pack was built from")
+        if index.dim() != 1 or index.shape[0] != B:
+            raise ValueError(f"shape mismatch: pred_cost {tuple(pred_cost.shape)}, index {tuple(index.shape)}")
+        idx = _to_device(index.detach(), dev, torch.int32)
+    elif sparse:
+        dev = _device_of(ctrs.val, device)
+        m, d = int(ctrs.m_max), int(ctrs.d)
+        if ctrs.batch != B:
+            raise ValueError(f"shape mismatch: pred_cost {tuple(pred_cost.shape)}, SparseConstraints of {ctrs.batch} instances")
+    else:
+        if ctrs is None:
+            raise ValueError("tight_ctrs is None and no pack= was given")
+        if ctrs.dim() != 3 or ctrs.shape[0] != B:
+            raise ValueError(f"shape mismatch: pred_cost {tuple(pred_cost.shape)}, tight_ctrs {tuple(ctrs.shape)}")
+        dev = _device_of(ctrs if ctrs.is_cuda else pred_cost, device)
+        _, m, d = ctrs.shape
+        ctrs = ctrs.detach()
+        if m == 0:      # no rows at all: behave like all-padding (src/cave.py:304-305)
+            ctrs, m = torch.zeros((B, 1, d), dtype=torch.float32, device=dev), 1
+        ctrs = _to_device(ctrs, dev, torch.float32) if ctrs.is_cuda else ctrs.to(torch.float32).contiguous()
+    if pred_cost.shape[1] != d:
+        raise ValueError(f"shape mismatch: pred_cost {tuple(pred_cost.shape)}, d = {d}")
+    io_dtype = torch.float64 if pred_cost.dtype == torch.float64 else torch.float32
+    io_code = _lib.F64 if io_dtype == torch.float64 else _lib.F32
+    compute = _PRECISIONS[precision]
+    host_out = not pred_cost.is_cuda
+    pred = pred_cost.detach()
+    pred = _to_device(pred, dev, io_dtype) if pred.is_cuda else pred.to(io_dtype).contiguous()
+    mr = _to_device(m_rows, dev, torch.int32) if (m_rows is not None and not resident) else None
+    bounds = chunk_bounds(B, chunk)
+    cap = max(hi - lo for lo, hi in bounds)
+    nb = ctypes.c_size_t()
+
+    with torch.cuda.device(dev):
+        cur = torch.cuda.current_stream(dev)
+        h2d, d2h = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
+        rings = {}
+        if not pred.is_cuda:
+            rings["pred"] = _Ring(pred, cap, dev)
+        if sparse:
+            sc_dev = ctrs.val.is_cuda
+            io_ = ctrs.inst_off.to(dev if sc_dev else "cpu", torch.int64).contiguous()
+            rp_ = ctrs.row_ptr.to(dev if sc_dev else "cpu", torch.int64).contiguous()
+            col_ = ctrs.col.to(dev if sc_dev else "cpu", torch.int32).contiguous()
+            val_ = ctrs.val.to(dev if sc_dev else "cpu", torch.float32).contiguous()
+            if not sc_dev:
+                rows = [(int(io_[lo]), int(io_[hi])) for lo, hi in bounds]
+                nnz = [(int(rp_[r0]), int(rp_[r1])) for r0, r1 in rows]
+                rings["inst_off"] = _Ring(io_, cap + 1, dev)
+                rings["row_ptr"] = _Ring(rp_, max(r1 - r0 for r0, r1 in rows) + 1, dev)
+                rings["col"] = _Ring(col_, max(z1 - z0 for z0, z1 in nnz), dev)
+                rings["val"] = _Ring(val_, max(z1 - z0 for z0, z1 in nnz), dev)
+            local_idx = torch.arange(cap, dtype=torch.int32, device=dev)
+        elif not resident and not ctrs.is_cuda:
+            rings["A"] = _Ring(ctrs, cap, dev)
+
+        # one pack and one scratch for the largest chunk, reused by every chunk (they run in order on the current stream)
+        opts0 = _opts(**solver)
+        _lib.check(lib.cave_scratch_bytes(cap, m, d, compute, ctypes.byref(opts0), ctypes.byref(nb)))
+        scratch = torch.empty(nb.value, dtype=torch.uint8, device=dev)
+        if resident:
+            pack_buf = pack.buf
+        else:
+            _lib.check(lib.cave_pack_bytes(cap, m, d, ctypes.byref(nb)))
+            pack_buf = torch.empty(nb.value, dtype=torch.uint8, device=dev)
+        _lib.check(lib.cave_chunk_acc_bytes(B, ctypes.byref(nb)))
+        acc = torch.empty(nb.value, dtype=torch.uint8, device=dev)
+        grad = torch.empty((B, d), dtype=io_dtype, device=dev) if not host_out else None
+        proj = torch.empty((B, d), dtype=io_dtype, device=dev) if (want_proj and not host_out) else None
+        if host_out:        # the chunks' outputs pass through two device buffers into pinned host memory
+            grad_h = torch.empty((B, d), dtype=io_dtype, pin_memory=True)
+            proj_h = torch.empty((B, d), dtype=io_dtype, pin_memory=True) if want_proj else None
+            out_stage = [torch.empty((2, cap, d), dtype=io_dtype, device=dev) for _ in range(2 if want_proj else 1)]
+        warm = ndense = gram = None
+        if resident:
+            warm, ndense, gram = pack.warm, pack.warm_dense, pack.gram
+        stream = ctypes.c_void_p(cur.cuda_stream)
+        copied = [torch.cuda.Event(), torch.cuda.Event()]       # on h2d: the inputs of the chunk in set s are on the device
+        computed = [torch.cuda.Event(), torch.cuda.Event()]     # on cur: the chunk in set s is solved (its inputs are free)
+        drained = [torch.cuda.Event(), torch.cuda.Event()]      # on d2h: the outputs of the chunk in set s reached the host
+        staged = [None, None]
+
+        def stage(k):
+            lo, hi = bounds[k]
+            s = k & 1
+            got = {}
+            with torch.cuda.stream(h2d):
+                h2d.wait_event(computed[s])
+                for name in ("pred", "A"):
+                    if name in rings:
+                        got[name] = rings[name].put(s, lo, hi, copied[s])
+                if sparse and not sc_dev:
+                    (r0, r1), (z0, z1) = rows[k], nnz[k]
+                    got["inst_off"] = rings["inst_off"].put(s, lo, hi + 1, copied[s])
+                    got["row_ptr"] = rings["row_ptr"].put(s, r0, r1 + 1, copied[s])
+                    got["col"] = rings["col"].put(s, z0, z1, copied[s])
+                    got["val"] = rings["val"].put(s, z0, z1, copied[s])
+                    _lib.check(lib.cave_csr_rebase(_ptr(got["inst_off"]), hi - lo + 1, r0, _ptr(got["row_ptr"]), r1 - r0 + 1,
+                                                   z0, ctypes.c_void_p(h2d.cuda_stream)))
+                copied[s].record(h2d)
+            staged[s] = got
+
+        stage(0)
+        for k, (lo, hi) in enumerate(bounds):
+            s, n = k & 1, hi - lo
+            got = staged[s]
+            cur.wait_event(copied[s])
+            p_pred = got["pred"] if "pred" in got else pred[lo:hi]
+            if host_out:
+                cur.wait_event(drained[s])
+                g_k = out_stage[0][s][:n]
+                p_k = out_stage[1][s][:n] if want_proj else None
+            else:
+                g_k, p_k = grad[lo:hi], (proj[lo:hi] if want_proj else None)
+            if resident:
+                A_k = A
+                opts = _opts(**solver, warm=True, index=idx[lo:hi], n_packed=N)
+            elif sparse:
+                if sc_dev:      # absolute offsets into the whole CSR, which is on the device
+                    io_k, rp_k, col_k, val_k = io_[lo:], rp_, col_, val_
+                else:
+                    io_k, rp_k, col_k, val_k = got["inst_off"], got["row_ptr"], got["col"], got["val"]
+                _lib.check(lib.cave_pack_sparse(_ptr(io_k), _ptr(rp_k), _ptr(col_k), _ptr(val_k), n, m, d, 0, _ptr(pack_buf),
+                                                pack_buf.numel(), stream))
+                A_k = None
+                opts = _opts(**solver, warm=True, index=local_idx[:n], n_packed=n)
+            else:
+                A_k = got["A"] if "A" in got else ctrs[lo:hi]
+                opts = _opts(**solver)
+            _lib.check(lib.cave_forward_backward_chunk(
+                _ptr(A_k), _ptr(mr[lo:hi] if mr is not None else None), _ptr(p_pred), n, m, d, float(sign), int(mode),
+                float(inner_ratio), _lib.REDUCE[reduction], io_code, compute, ctypes.byref(opts), None, None, _ptr(g_k),
+                _ptr(p_k), None, None, None, _ptr(pack_buf), pack_buf.numel(), _ptr(scratch), scratch.numel(),
+                _ptr(warm), warm.numel() if warm is not None else 0, _ptr(ndense), ndense.numel() if ndense is not None else 0,
+                _ptr(gram), gram.numel() if gram is not None else 0, lo, B, _ptr(acc), acc.numel(), stream))
+            computed[s].record(cur)
+            if host_out:
+                with torch.cuda.stream(d2h):
+                    d2h.wait_event(computed[s])
+                    grad_h[lo:hi].copy_(g_k, non_blocking=True)
+                    if want_proj:
+                        proj_h[lo:hi].copy_(p_k, non_blocking=True)
+                    drained[s].record(d2h)
+            if k + 1 < len(bounds):
+                stage(k + 1)        # after the launches of chunk k: a pageable host copy overlaps its solve
+        cur.wait_stream(h2d)
+        cur.wait_stream(d2h)
+        for t in [*(r.dev for r in rings.values())]:
+            for b in t:
+                b.record_stream(h2d)
+        if host_out:
+            for t in out_stage:
+                t.record_stream(d2h)
+
+        loss = torch.empty((), dtype=io_dtype, device=dev)
+        loss_i = torch.empty(B, dtype=io_dtype, device=dev)
+        rnorm = torch.empty(B, dtype=io_dtype, device=dev) if (want_proj or want_status) else None
+        status = torch.empty(B, dtype=torch.int32, device=dev) if want_status else None
+        iters = torch.empty(B, dtype=torch.int32, device=dev) if want_status else None
+        _lib.check(lib.cave_chunk_finalize(_ptr(acc), acc.numel(), B, _lib.REDUCE[reduction], io_code, _ptr(loss), _ptr(loss_i),
+                                           _ptr(rnorm), _ptr(status), _ptr(iters), stream))
+        out = dict(loss=loss_i if reduction == "none" else loss, loss_i=loss_i, grad=grad)
+        if want_proj:
+            out["proj"], out["rnorm"] = proj, rnorm
+        if want_status:
+            out["status"], out["iters"], out["rnorm"] = status, iters, rnorm
+        if host_out:
+            for key, v in out.items():
+                if v is not None and key not in ("grad", "proj"):
+                    h = torch.empty(v.shape, dtype=v.dtype, pin_memory=True)
+                    h.copy_(v, non_blocking=True)
+                    out[key] = h
+            out["loss"] = out["loss_i"] if reduction == "none" else out["loss"]
+            out["grad"] = grad_h
+            if want_proj:
+                out["proj"] = proj_h
+            cur.synchronize()
     return out
 
 

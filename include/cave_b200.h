@@ -194,7 +194,9 @@ int cave_forward_backward(const float* A, const int32_t* m_rows, const void* pre
  *    instances, heuristic mode, empty cones, NaN / Inf predictions and instances with more variables than a slot holds
  *    leave it untouched.
  *  - Calls that share one buffer must be ordered (one stream), as calls that share a pack or scratch are.  An index may
- *    hold an instance twice: the slot is then read and written concurrently, which can only change the starting guess. */
+ *    hold an instance twice: the slot is then read and written concurrently, which can only change the starting guess.
+ *    Across the chunks of a chunked batch (cave_forward_backward_chunk) the order is fixed instead: an instance in two
+ *    chunks is read by the later chunk after the earlier one wrote it, so it can start from that solution. */
 int cave_warm_bytes(int64_t n_instances, int64_t m_max, int64_t d, size_t* out);
 int cave_forward_backward_warm(const float* A, const int32_t* m_rows, const void* pred,
                                int64_t B, int64_t m_max, int64_t d,
@@ -269,6 +271,44 @@ int cave_forward_backward_resident(const float* A, const int32_t* m_rows, const 
                                    void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
                                    void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
                                    const void* gram, size_t gram_bytes, void* stream);
+
+/* Chunked calls: one batch of batch_total rows solved as consecutive chunks, so that device memory scales with the chunk
+ * and the host-device copies of one chunk can overlap the solve of another (cave_b200.qpsolver, `chunk=`).  Every instance
+ * is solved independently, so a chunked batch gives the unchunked call's per-instance results; the reduced loss is the
+ * unchunked one bit for bit because cave_chunk_finalize() reduces the whole batch in the same fixed order.
+ * cave_chunk_acc_bytes(): bytes of the caller-owned whole-batch accumulator, four arrays each starting 256-byte aligned:
+ *   float64 loss[B_total], float64 rnorm[B_total], int32 status[B_total], int32 iters[B_total].
+ * cave_forward_backward_chunk(): cave_forward_backward_resident for batch rows [batch_offset, batch_offset + B) of the batch:
+ *  - pred, grad and proj (and inst_index, m_rows) point at this chunk's rows; the per-instance float64 loss / rnorm and the
+ *    status / iters words go to acc at batch_offset; loss, loss_i, rnorm, status and iters are not written (may be null);
+ *  - for CAVE_REDUCE_MEAN the gradient scale is 1 / batch_total;
+ *  - warm, warm_dense and gram may each be null, all three included; without opts->warm_pack the chunk's rows of A get a
+ *    one-shot pack as in cave_forward_backward;
+ *  - CAVE_EINVAL: batch_offset < 0, batch_offset + B > batch_total, null or not 256-byte aligned acc; CAVE_ELIMIT:
+ *    batch_total above the batch limit; CAVE_ENOSPC: acc_bytes < cave_chunk_acc_bytes(batch_total).
+ * Chunks of one batch may run in any order but on one stream (they share pack and scratch), as may their warm-start
+ * slots: a chunk's writes to a slot come before a later chunk's reads of it.
+ * cave_chunk_finalize(): after the last chunk, the reduction and dtype conversion of cave_forward_backward over the whole
+ * accumulator: loss (MEAN / SUM; may be null for NONE), loss_i [batch_total] (required), rnorm, status, iters (optional). */
+int cave_chunk_acc_bytes(int64_t B_total, size_t* out);
+int cave_forward_backward_chunk(const float* A, const int32_t* m_rows, const void* pred,
+                                int64_t B, int64_t m_max, int64_t d,
+                                double sign, int mode, double inner_ratio, int reduction,
+                                int io_dtype, int compute_dtype, const cave_solver_opts* opts,
+                                void* loss, void* loss_i, void* grad, void* proj, void* rnorm,
+                                int32_t* status, int32_t* iters,
+                                void* pack, size_t pack_bytes, void* scratch, size_t scratch_bytes,
+                                void* warm, size_t warm_bytes, void* warm_dense, size_t warm_dense_bytes,
+                                const void* gram, size_t gram_bytes,
+                                int64_t batch_offset, int64_t batch_total, void* acc, size_t acc_bytes, void* stream);
+int cave_chunk_finalize(const void* acc, size_t acc_bytes, int64_t batch_total, int reduction, int io_dtype,
+                        void* loss, void* loss_i, void* rnorm, int32_t* status, int32_t* iters, void* stream);
+
+/* Rebases, in place on the device, a chunk of per-instance CSR (cave_pack_sparse) cut out of a larger one: subtracts
+ * row_base from inst_off[0 .. n_inst_off) and nnz_base from row_ptr[0 .. n_row_ptr), so that the chunk's offsets start at
+ * zero (row_base = the batch's inst_off at the chunk's first instance, nnz_base = its row_ptr at that row). */
+int cave_csr_rebase(int64_t* inst_off, int64_t n_inst_off, int64_t row_base, int64_t* row_ptr, int64_t n_row_ptr,
+                    int64_t nnz_base, void* stream);
 
 /* Diagnostic for the dense regime (north_star item 1): runs cave_pack() on A and then only the TF32 split and the
  * tensor-core Gram kernel (TMA tiles -> tcgen05.mma, 3xTF32, float32 accumulation in TMEM) for the first
